@@ -7,6 +7,9 @@
 A step = one `_update_step` (rec_magpo.py:106-499): T env steps of U*E envs through guider + learner + env,
 GAE, then P epochs x M minibatches of guider/learner forward+backward, the gradient all-reduce and clip+Adam.
 Metric: agent-env-steps/s = n_gpus * U * E * T * A / step time (whole job). Weak scaling: E per GPU is fixed.
+Every warm-up and timed step starts from the same seeded learner state, restored before the step and outside its timed span: the
+update sums gradients with float atomics, so the parameters of consecutive steps drift apart between runs in the last bits, and the
+next rollout's sampling turns that into different trajectories. From one state, two runs compute the same step up to rounding.
 Prints ONE JSON line on rank 0.
 """
 from __future__ import annotations
@@ -59,7 +62,16 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-profile", action="store_true")
     ap.add_argument("--quick", action="store_true", help="1 warm-up step, no e2e loop (for runs under ncu only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (episode metrics, loss sums) and the learner state it left "
+                         "(parameters, step key, hidden states) as DIR/<name>.npy; arrays above 2^20 elements are replaced by "
+                         "the same seeded sample of 2^20 of them on every run")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def workload_config(args, n_gpus):
@@ -133,6 +145,38 @@ def run_reference(args, as_baseline=False):
     return val, dt, cores, sample, E, warm
 
 
+DUMP_MAX_ELEMENTS = 1 << 20  # 4 MB per array: the 11 arrays of step_outputs stay under 64 MB at any size
+
+
+def learner_snapshot(lrn):
+    """(buffer, saved copy) pairs of everything an update step reads that an earlier step wrote: parameters, Adam state, step key,
+    env state and timestep, recurrent states, and the trajectory's last observation slot, which the next rollout carries over into
+    slot 0. Taken right after `reset`, that slot gets the reset observation of slot 0."""
+    T = lrn.sys.rollout_length
+    pairs = [(t, t.clone()) for t in (lrn.guider, lrn.actor, lrn.g_mu, lrn.g_nu, lrn.a_mu, lrn.a_nu, lrn.g_count, lrn.a_count,
+                                      lrn.key, lrn.policy_h, *lrn.env_state.values(), *lrn.ts.values(), *lrn.hs.values())]
+    pairs += [(lrn.traj[k][T], lrn.traj[k][0].clone()) for k in ("done", "agents_view", "action_mask", "step_count")]
+    return pairs
+
+
+def step_outputs(lrn, metrics, losses):
+    """Host copies of what one `update_step` hands its caller: the episode metrics and loss sums it returns, and the learner
+    state it leaves (flat parameter buffers, step key, recurrent states). float32, the key as float64 (uint32 values)."""
+    import numpy as np
+    import torch
+
+    arrays = {**metrics, "losses": losses, "guider_params": lrn.guider, "actor_params": lrn.actor, "policy_hidden_state": lrn.policy_h,
+              **{f"sable_hidden_state_{k}": v for k, v in lrn.sable_hidden_state().items()}}
+    out = {}
+    for name, t in arrays.items():
+        if t.numel() > DUMP_MAX_ELEMENTS:  # a flat, seeded sample: the same elements on every run with the same arguments
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMENTS, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        out[name] = t.float().cpu().numpy()
+    out["key"] = lrn.key.cpu().numpy().view(np.uint32).astype(np.float64)
+    return out
+
+
 def main():
     # stdout carries exactly ONE line (the JSON): everything else that native libraries print there (e.g. NCCL's version
     # banner) is routed to stderr while the benchmark runs
@@ -204,26 +248,37 @@ def run():
             comm.barrier()
         torch.cuda.synchronize()
 
+    snapshot = learner_snapshot(lrn)
+
+    def restore():
+        for buf, saved in snapshot:
+            buf.copy_(saved)
+
     def timed(fn, k):
+        """(ms per call, what the last call returned); the learner state is restored before each call, outside its span"""
         barrier()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(k):
-            fn()
-        e1.record()
+        spans = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(k)]
+        for e0, e1 in spans:
+            restore()
+            e0.record()
+            last = fn()
+            e1.record()
         barrier()
-        ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
+        ms = torch.tensor([sum(e0.elapsed_time(e1) for e0, e1 in spans)], device=dev)
         if comm is not None:
             comm.allreduce_max(ms)
-        return float(ms.item()) / k
+        return float(ms.item()) / k, last
 
     for _ in range(1 if args.quick else max(3, args.warmup)):
+        restore()
         lrn.update_step()
     sampler = ClockSampler(local_rank)
     sampler.start()
     n0 = lib.magpo_launch_count()
-    ms = timed(lrn.update_step, args.steps)
+    ms, last = timed(lrn.update_step, args.steps)
     launches = lib.magpo_launch_count() - n0
+    # the steps below overwrite the learner's buffers: copy the last timed step's outputs out first
+    dump = step_outputs(lrn, *last) if args.dump_outputs and rank == 0 else None
 
     # end to end through the public call, host buffers: per step the step key goes up from pinned memory and the
     # metrics the experiment loop consumes (episode metrics [T,B], the [P,M,8] loss sums, the new key) come back.
@@ -246,7 +301,7 @@ def run():
         key_host.copy_(lrn.key, non_blocking=True)
         torch.cuda.current_stream().synchronize()  # the host reads the metrics every step
 
-    ms_e2e = ms if args.quick else timed(e2e_step, args.steps)
+    ms_e2e = ms if args.quick else timed(e2e_step, args.steps)[0]
     sampler.stop_flag = True
     sampler.join(timeout=2)
 
@@ -258,6 +313,7 @@ def run():
 
     # phase split of one more step (CUDA events on the launching stream)
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
+    restore()
     torch.cuda.synchronize()
     ev[0].record(); lrn.rollout(); ev[1].record(); lrn.gae(); ev[2].record()
     for p_ in range(sysc.ppo_epochs):
@@ -279,6 +335,7 @@ def run():
         lib.magpo_prof_enable(1 if rank == 0 else 0)
         lrn.graph_rollout = False  # the per-category events are recorded by eager launches, not by a graph replay
         lib.magpo_debug_set_overlap(0)  # ... and kernel by kernel: no guider/learner stream overlap inside this step
+        restore()
         lrn.update_step()
         torch.cuda.synchronize()
         lib.magpo_debug_set_overlap(1)
@@ -350,6 +407,10 @@ def run():
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         val, dt, cores, sample, _, _ = run_reference(args, as_baseline=True)
         out["cpu_baseline"] = {"value": val, "unit": UNIT, "cores": cores, "kind": "port", "sample": sample}
+    if dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dump.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
     if comm is not None:
         comm.barrier()
         comm.close()

@@ -4,6 +4,10 @@ The reference ships no golden vectors and cannot be imported here (JAX is absent
 fixtures pin the ORACLE's current outputs (regression anchors shared by the CPU and the GPU tests); the
 published Random123 / jax.random KATs are asserted separately in tests/test_oracle.py.
 Run from the repo root:  python tests/golden/make_golden.py
+
+    python tests/golden/make_golden.py --reference <liyheng/MAGPO checkout>
+rewrites only reference_configs.json: the reference's env and scenario YAML fields that the in-tree config tree
+(magpo_b200/configs/env) and the oracle's scenario tables must carry.
 """
 import json
 import os
@@ -95,5 +99,30 @@ def env_trace(mod, spec, n_steps, n_envs=6, seed=9):
                 final_key=st["env_state"]["key"])
 
 
+def reference_configs(env_dir):
+    """{"env": {family: env_name / kwargs / defaults}, "scenario": {file stem: name / task_name / task_config}} of a
+    mava/configs/env tree."""
+    import glob
+
+    import yaml
+
+    env = {}
+    for fam in ("coordsum", "lbf", "rware"):
+        with open(os.path.join(env_dir, f"{fam}.yaml")) as f:
+            y = yaml.safe_load(f)
+        env[fam] = {k: y[k] for k in ("env_name", "kwargs", "defaults")}
+    scenario = {}
+    for path in sorted(glob.glob(os.path.join(env_dir, "scenario", "*.yaml"))):
+        with open(path) as f:
+            y = yaml.safe_load(f)
+        scenario[os.path.basename(path)[:-len(".yaml")]] = {k: y[k] for k in ("name", "task_name", "task_config")}
+    return {"env": env, "scenario": scenario}
+
+
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) == 3 and sys.argv[1] == "--reference":
+        with open(os.path.join(HERE, "reference_configs.json"), "w") as f:
+            json.dump(reference_configs(os.path.join(sys.argv[2], "mava", "configs", "env")), f, indent=1)
+            f.write("\n")
+    else:
+        main()

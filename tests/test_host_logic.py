@@ -139,21 +139,21 @@ def test_checkpointer_keeps_the_best_and_restores(tmp_path, monkeypatch):
 
 def test_env_scenario_files_match_the_reference_configs():
     """Every LBF / RWARE / CoordSum scenario file shipped here carries the reference's `task_config` (mava/configs/env/scenario/*.yaml);
-    skipped where the reference tree is absent (the GPU box)."""
+    the reference's values are stored in tests/golden/reference_configs.json (make_golden.py --reference)."""
     import glob
+    import json
     import os
 
-    import pytest
     import yaml
 
-    ref_dir = "/root/reference/mava/configs/env/scenario"
-    if not os.path.isdir(ref_dir):
-        pytest.skip("reference tree not present")
-    here = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "magpo_b200", "configs", "env", "scenario")
+    tests = os.path.dirname(os.path.abspath(__file__))
+    with open(os.path.join(tests, "golden", "reference_configs.json")) as f:
+        gold = json.load(f)
+    here = os.path.join(os.path.dirname(tests), "magpo_b200", "configs", "env", "scenario")
     checked = 0
     for path in glob.glob(os.path.join(here, "*.yaml")):
         mine = yaml.safe_load(open(path))
-        ref = yaml.safe_load(open(os.path.join(ref_dir, os.path.basename(path))))
+        ref = gold["scenario"][os.path.basename(path)[:-len(".yaml")]]
         assert mine["task_name"] == ref["task_name"] and mine["name"] == ref["name"], path
         for k, v in ref["task_config"].items():
             assert mine["task_config"][k] == v, (path, k)
@@ -161,7 +161,7 @@ def test_env_scenario_files_match_the_reference_configs():
     assert checked >= 20
     for env in ("lbf", "rware", "coordsum"):
         mine = yaml.safe_load(open(os.path.join(os.path.dirname(here), f"{env}.yaml")))
-        ref = yaml.safe_load(open(f"/root/reference/mava/configs/env/{env}.yaml"))
+        ref = gold["env"][env]
         assert mine["env_name"] == ref["env_name"] and mine["kwargs"] == ref["kwargs"] and mine["defaults"] == ref["defaults"], env
 
 

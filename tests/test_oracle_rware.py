@@ -1,8 +1,10 @@
 """CPU: the RobotWarehouse restatement (oracle/rware.py) against hand-computed cases and generator invariants.
 These pin the restatement, not a Jumanji run (parity unpinned, see the oracle's header)."""
+import json
+import os
+
 import numpy as np
 import pytest
-import yaml
 
 from oracle import prng, rware
 
@@ -23,13 +25,11 @@ def _place(spec, e, agent, pos, direction, carry=False):
 
 
 def test_layouts_and_scenarios_match_the_reference_configs():
+    # the reference's mava/configs/env/scenario/*.yaml, as stored by tests/golden/make_golden.py --reference
+    with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_configs.json")) as f:
+        ref = json.load(f)["scenario"]
     for name, kw in rware.SCENARIOS.items():
-        path = f"/root/reference/mava/configs/env/scenario/{name}.yaml"
-        try:
-            y = yaml.safe_load(open(path))
-        except FileNotFoundError:  # the reference tree is absent on the GPU box
-            continue
-        assert y["task_config"] == kw, name
+        assert ref[name]["task_config"] == kw, name
     tiny, small = rware.RwareSpec(**rware.SCENARIOS["tiny-4ag"]), rware.RwareSpec(**rware.SCENARIOS["small-4ag"])
     assert tiny.grid_size == (11, 10) and len(tiny.shelf_cells) == 32 and tiny.obs_dim == 75 and tiny.goals == [(10, 4), (10, 5)]
     assert small.grid_size == (20, 10) and len(small.shelf_cells) == 80
