@@ -218,3 +218,31 @@ extern "C" int magpo_debug_force_gru_stepwise(int on) {
   magpo::g_force_stepwise = on != 0;
   return MAGPO_OK;
 }
+
+// Test hook: the persistent GRU scans on caller buffers, set up as actor_forward / actor_backward set them up.
+//   gi [T, Rs, 384] (x @ Wi + bi), Wh [128, 384], bhn [128], done [T, N], h0 [Rs, 128], dY [T, Rs, 128]; Rs = N * A.
+//   scratch: 3 * 128 * 384 floats (W_h^T and the TF32 hi / lo images).
+//   bwd == 0: HU[0] = h0 masked by done[0], then rzn [T, Rs, 384], ghn / Y [T, Rs, 128], HU [T+1, Rs, 128].
+//   bwd != 0: from the forward's rzn / ghn / HU: dgi, dgh [T, Rs, 384]; dbi [384] and dbhn [128] are accumulated into.
+// There is no stepwise fallback here: MAGPO_ERR_UNSUPPORTED when the tensor-core path is off or T < 2.
+extern "C" int magpo_test_gru_scan(magpo_stream_t s_, int bwd, int T, int N, int A, const float* gi, const float* Wh,
+                                   const float* bhn, const uint8_t* done, const float* h0, const float* dY, float* scratch,
+                                   float* rzn, float* ghn, float* Y, float* HU, float* dgi, float* dgh, float* dbi, float* dbhn) {
+  using namespace magpo;
+  if (!tc_enabled() || T < 2) return MAGPO_ERR_UNSUPPORTED;
+  if (N < 1 || A < 1 || !gi || !Wh || !done || !scratch || !rzn || !ghn || !HU) return MAGPO_ERR_ARG;
+  cudaStream_t s = as_stream(s_);
+  const int64_t Rs = (int64_t)N * A, n = 3 * kH * kH;
+  float *hi = scratch + n, *lo = scratch + 2 * n;
+  if (!bwd) {
+    if (!bhn || !h0 || !Y) return MAGPO_ERR_ARG;
+    mask_rows_kernel<<<g256(Rs * kH), 256, 0, s>>>(Rs, A, h0, done, HU);
+    MAGPO_LAUNCH_OK();
+    MAGPO_TRY(transpose(s, kH, 3 * kH, Wh, scratch));
+    MAGPO_TRY(tc_prepare_region(s, scratch, n, hi, lo));
+    return gru_scan_fwd(s, T, N, A, gi, hi, lo, bhn, done, rzn, ghn, Y, HU);
+  }
+  if (!dY || !dgi || !dgh) return MAGPO_ERR_ARG;
+  MAGPO_TRY(tc_prepare_region(s, Wh, n, hi, lo));
+  return gru_scan_bwd(s, T, N, A, dY, rzn, ghn, HU, done, hi, lo, dgi, dgh, dbi, dbhn);
+}

@@ -738,3 +738,6 @@ extern "C" int magpo_debug_gru_timeline(unsigned long long* buf) {
   magpo::g_gru_dbg = buf;
   return MAGPO_OK;
 }
+
+// Host-only: the rows per CTA both scans launch with for Rs = N * A rows (tests assert which tile branch a case covers).
+extern "C" int magpo_debug_gru_rows_per_tile(int64_t Rs) { return magpo::gru_rows_per_tile(Rs); }

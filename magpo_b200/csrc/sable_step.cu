@@ -674,16 +674,19 @@ int launch_ae(cudaStream_t st, const GuiderP& p, const StepArgs& s) {
   return MAGPO_OK;
 }
 
-template <int A>
-int launch_a(cudaStream_t st, const GuiderP& p, const StepArgs& s) {
-  // envs per warp: 2 when the batch fills the 296 CTA slots anyway, 1 below that (twice the warps, half the chain per warp)
+// envs per warp: 2 when the batch fills the 296 CTA slots anyway, 1 below that (twice the warps, half the chain per warp)
+int envs_per_warp(int64_t B) {
   static int forced_epw = -1;
   if (forced_epw < 0) {
     const char* e = getenv("MAGPO_STEP_EPW");
     forced_epw = e ? atoi(e) : 0;
   }
-  const int epw = (forced_epw == 1 || forced_epw == 2) ? forced_epw : (s.B <= 2048 ? 1 : 2);
-  return epw == 1 ? launch_ae<A, 1>(st, p, s) : launch_ae<A, 2>(st, p, s);
+  return (forced_epw == 1 || forced_epw == 2) ? forced_epw : (B <= 2048 ? 1 : 2);
+}
+
+template <int A>
+int launch_a(cudaStream_t st, const GuiderP& p, const StepArgs& s) {
+  return envs_per_warp(s.B) == 1 ? launch_ae<A, 1>(st, p, s) : launch_ae<A, 2>(st, p, s);
 }
 
 }  // namespace
@@ -732,3 +735,12 @@ int sable_step(cudaStream_t st, const MagpoNetCfg* net, int B, int gumbel_rows, 
 }
 
 }  // namespace magpo
+
+// Host-only: the envs per warp and warps per CTA the fused step kernel launches with for B envs (tests assert which branch a case
+// covers).
+extern "C" int magpo_debug_step_plan(int32_t B, int32_t* epw, int32_t* warps) {
+  if (B < 1 || !epw || !warps) return MAGPO_ERR_ARG;
+  *epw = magpo::envs_per_warp(B);
+  *warps = magpo::pick_warps(magpo::ceil_div(B, *epw));
+  return MAGPO_OK;
+}
