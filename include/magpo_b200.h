@@ -8,7 +8,8 @@
  *   - the CUDA stream (cudaStream_t passed as void*) comes first, after the per-device MagpoContext* for the entry points that
  *     need one (see below); all work is enqueued on that stream (forked context streams are joined back before the call
  *     returns), nothing synchronises, nothing allocates: every buffer is a caller-owned DEVICE pointer, scratch is passed
- *     explicitly and sized by the matching *_workspace_bytes(); there is no process-global state;
+ *     explicitly and sized by the matching *_workspace_bytes(); there is no process-global state on the product path (the
+ *     benchmark / test hooks magpo_prof_*, magpo_debug_set_overlap and magpo_set_chain_kernels are process-wide; it never sets them);
  *   - POD attribute structs by const pointer; no torch / C++ types in any signature;
  *   - return 0 on success, a negative MAGPO_ERR_* otherwise (no exceptions cross the ABI);
  *   - single host thread per device (the reference path is single-threaded).
@@ -43,7 +44,8 @@ const char* magpo_last_cuda_error(void);
  * Per-device context, created by the caller and passed to every entry point that needs more than its arguments: the entry points that
  * fork work onto side streams (rollout, minibatch_grads, guider_forward) or that look up the TF32 images of weight matrices they
  * prepared in the caller's workspace (all GEMM users). It owns three non-blocking streams with their fork / join events and a
- * host-side table of prepared weight regions; nothing in the library is process-global, so several learners — on the same device
+ * host-side table of prepared weight regions; nothing the product path uses is process-global (only the benchmark / test hooks
+ * magpo_prof_*, magpo_debug_set_overlap and magpo_set_chain_kernels are, and it never sets them), so several learners — on the same device
  * or on different ones — can be driven from one process and interleaved freely. A context is bound to the device it was created
  * on: calling with another device current returns MAGPO_ERR_ARG. One host thread at a time per context. The remaining entry points
  * (PRNG, envs, GAE, shuffle / pack, clip+Adam) are stateless and take no context. */

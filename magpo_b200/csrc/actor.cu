@@ -82,8 +82,6 @@ inline unsigned g256(int64_t n) { return (unsigned)ceil_div(n, 256); }
 
 }  // namespace
 
-bool g_force_stepwise = false;  // tests / tools: A/B the persistent scans against the per-timestep GEMM + gate kernels
-
 void ActorT::plan(Arena& ar, int a) {
   WiT = ar.get<float>(3 * kH * kH);
   WhT = ar.get<float>(3 * kH * kH);
@@ -99,7 +97,7 @@ int actor_transpose(cudaStream_t s, const ActorP& p, const ActorT& t, int a) {
   MAGPO_TRY(transpose(s, kH, 3 * kH, p.Wh, t.WhT));
   MAGPO_TRY(transpose(s, kH, kH, p.post_w, t.postT));
   MAGPO_TRY(transpose(s, kH, a, p.head_w, t.headT));
-  if (tc_enabled()) MAGPO_TRY(tc_prepare_region(s, t.WiT, t.region_n, t.region_hi, t.region_lo));
+  MAGPO_TRY(tc_prepare_region(s, t.WiT, t.region_n, t.region_hi, t.region_lo));
   return MAGPO_OK;
 }
 
@@ -137,7 +135,7 @@ int actor_forward(cudaStream_t s, const ActorP& p, const ActorT* pt, int T, int 
     MAGPO_LAUNCH_OK();
   }
   const float *wh_hi = nullptr, *wh_lo = nullptr;
-  const bool scan = T > 1 && w.rzn && pt && tc_enabled() && !g_force_stepwise && tc_lookup(pt->WhT, &wh_hi, &wh_lo);
+  const bool scan = T > 1 && w.rzn && pt && tc_lookup(pt->WhT, &wh_hi, &wh_lo);
   if (scan) MAGPO_TRY(gru_scan_fwd(s, T, N, A, w.gi, wh_hi, wh_lo, p.bhn, done, w.rzn, w.ghn, w.Y, w.HU));
   for (int t = 0; t < T && !scan; ++t) {
     const float* hu = mask_in_gate ? h0 : w.HU + (size_t)t * Rs * kH;
@@ -181,7 +179,7 @@ int actor_backward(cudaStream_t s, const ActorP& p, const ActorT& pt, int T, int
   // reverse scan; dgi reuses the gi buffer (dead after the forward)
   float* dgi = w.gi;
   const float *wh_hi = nullptr, *wh_lo = nullptr;
-  const bool scan = T > 1 && tc_enabled() && !g_force_stepwise && tc_lookup(p.Wh, &wh_hi, &wh_lo);
+  const bool scan = T > 1 && tc_lookup(p.Wh, &wh_hi, &wh_lo);
   if (scan) MAGPO_TRY(gru_scan_bwd(s, T, N, A, w.dB, w.rzn, w.ghn, w.HU, done, wh_hi, wh_lo, dgi, w.dgh, g.bi, g.bhn));  // bias sums inside
   for (int t = T - 1; t >= 0 && !scan; --t) {
     const size_t o1 = (size_t)t * Rs * kH, o3 = (size_t)t * Rs * 3 * kH;
@@ -214,22 +212,17 @@ int actor_backward(cudaStream_t s, const ActorP& p, const ActorT& pt, int T, int
 
 }  // namespace magpo
 
-extern "C" int magpo_debug_force_gru_stepwise(int on) {
-  magpo::g_force_stepwise = on != 0;
-  return MAGPO_OK;
-}
-
 // Test hook: the persistent GRU scans on caller buffers, set up as actor_forward / actor_backward set them up.
 //   gi [T, Rs, 384] (x @ Wi + bi), Wh [128, 384], bhn [128], done [T, N], h0 [Rs, 128], dY [T, Rs, 128]; Rs = N * A.
 //   scratch: 3 * 128 * 384 floats (W_h^T and the TF32 hi / lo images).
 //   bwd == 0: HU[0] = h0 masked by done[0], then rzn [T, Rs, 384], ghn / Y [T, Rs, 128], HU [T+1, Rs, 128].
 //   bwd != 0: from the forward's rzn / ghn / HU: dgi, dgh [T, Rs, 384]; dbi [384] and dbhn [128] are accumulated into.
-// There is no stepwise fallback here: MAGPO_ERR_UNSUPPORTED when the tensor-core path is off or T < 2.
+// There is no stepwise fallback here: MAGPO_ERR_UNSUPPORTED when T < 2.
 extern "C" int magpo_test_gru_scan(magpo_stream_t s_, int bwd, int T, int N, int A, const float* gi, const float* Wh,
                                    const float* bhn, const uint8_t* done, const float* h0, const float* dY, float* scratch,
                                    float* rzn, float* ghn, float* Y, float* HU, float* dgi, float* dgh, float* dbi, float* dbhn) {
   using namespace magpo;
-  if (!tc_enabled() || T < 2) return MAGPO_ERR_UNSUPPORTED;
+  if (T < 2) return MAGPO_ERR_UNSUPPORTED;
   if (N < 1 || A < 1 || !gi || !Wh || !done || !scratch || !rzn || !ghn || !HU) return MAGPO_ERR_ARG;
   cudaStream_t s = as_stream(s_);
   const int64_t Rs = (int64_t)N * A, n = 3 * kH * kH;

@@ -49,7 +49,8 @@ struct ProfScope {
 
 // ---- per-device context (MagpoContext of the C ABI): everything an entry point needs besides its arguments. Created by the caller
 // (magpo_context_create), passed to every entry point that forks streams or looks up tensor-core weight images; nothing of it is
-// process-global, so several learners (and several devices) can be driven from one process.
+// process-global, so several learners (and several devices) can be driven from one process. The only process-wide switches are the
+// benchmark / test hooks magpo_prof_*, magpo_debug_set_overlap and magpo_set_chain_kernels; the product path never sets them.
 struct ForkJoin {  // a forked stream + the events that fork it off / join it back into the caller's stream
   cudaStream_t s = nullptr;
   cudaEvent_t fork = nullptr, join = nullptr;

@@ -424,12 +424,6 @@ bool make_map(CUtensorMap* tm, const float* ptr, int64_t rows, int cols, int ld,
              swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-bool env_tc_default() {
-  const char* e = getenv("MAGPO_TENSOR_CORES");  // "0" forces the fp32 SIMT GEMMs everywhere
-  return !(e && e[0] == '0');
-}
-bool g_tc_enabled = env_tc_default();
-
 }  // namespace
 
 bool tc_make_map(void* tensor_map, const float* ptr, int64_t rows, int cols, int ld, int box_rows) {
@@ -448,8 +442,6 @@ bool tc_make_map3(void* tensor_map, const float* ptr, int64_t T, int64_t rows, i
              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
-void tc_set_enabled(bool on) { g_tc_enabled = on; }
-bool tc_enabled() { return g_tc_enabled; }
 
 // Split a weight region into TF32 hi/lo copies and remember the mapping so that GEMMs on any sub-matrix find them.
 int tc_prepare_region(cudaStream_t s, const float* base, int64_t n, float* hi, float* lo) {
@@ -489,13 +481,8 @@ bool tc_lookup(const float* w, const float** hi, const float** lo) {
 static bool tc_plan(int64_t M, int N, int K, TcParams* p, uint32_t* smem_bytes) {
   if (K % TC_KC || K < TC_KC || N % 32 || M < 1) return false;
   const int cands[] = {256, 192, 128, 96, 64, 32};
-  static int max_bn = -1;
-  if (max_bn < 0) {
-    const char* e = getenv("MAGPO_TC_MAX_BN");  // experiments: cap the N tile of the forward GEMM
-    max_bn = e ? atoi(e) : 256;
-  }
   for (int bn : cands) {
-    if (N % bn || bn > max_bn) continue;
+    if (N % bn) continue;
     const uint32_t b_bytes = (uint32_t)K * bn * 8;
     const uint32_t fixed = b_bytes + 2 * TC_CHUNK_BYTES + 256 * 4 + 256 + 1024 /*alignment slack*/;
     if (fixed + 2 * 2 * TC_CHUNK_BYTES > TC_SMEM_LIMIT) continue;
@@ -515,7 +502,7 @@ static bool tc_plan(int64_t M, int N, int K, TcParams* p, uint32_t* smem_bytes) 
 }
 
 bool tc_supported(int64_t M, int N, int K, const float* X, int ldx, const float* Y, int ldy, int ldb) {
-  if (!g_tc_enabled || !get_encode()) return false;
+  if (!get_encode()) return false;
   if ((ldx & 3) || (ldy & 3) || (ldb & 3)) return false;
   if ((reinterpret_cast<uintptr_t>(X) & 15) || (reinterpret_cast<uintptr_t>(Y) & 15)) return false;
   TcParams p;
@@ -550,19 +537,9 @@ int gemm_tc(cudaStream_t s, int64_t M, int N, int K, const float* X, int ldx, co
 static bool tn_plan(int N, int K, TnParams* p, uint32_t* smem_bytes) {
   if ((K != 64 && K != 128) || N % 32) return false;
   const int cands[] = {256, 192, 128, 96, 64, 32};
-  static int max_bn = -1;
-  if (max_bn < 0) {
-    const char* e = getenv("MAGPO_TN_MAX_BN");  // experiments: cap the N tile of the weight-gradient GEMM
-    max_bn = e ? atoi(e) : 256;
-  }
   for (int bn : cands) {
-    if (N % bn || bn > max_bn) continue;
-    static int rc_big = -1;
-    if (rc_big < 0) {
-      const char* e = getenv("MAGPO_TN_ROWS");  // experiments: 32 = always 32 rows per stage
-      rc_big = (e && atoi(e) == 32) ? 32 : 64;
-    }
-    const int rc = (K / 32 + bn / 32) <= 4 ? rc_big : 32;
+    if (N % bn) continue;
+    const int rc = (K / 32 + bn / 32) <= 4 ? 64 : 32;
     const uint32_t raw = (uint32_t)(K / 32 + bn / 32) * (uint32_t)rc * 128u;
     const uint32_t fixed = 2 * TC_CHUNK_BYTES + 256 + 1024;
     if (fixed + 2 * 2 * raw > TC_SMEM_LIMIT) continue;
@@ -580,7 +557,7 @@ static bool tn_plan(int N, int K, TnParams* p, uint32_t* smem_bytes) {
 }
 
 bool tc_tn_supported(int64_t M, int N, int K, const float* X, int ldx, const float* dY, int ldy, const float* dW, int ldw) {
-  if (!g_tc_enabled || !get_encode()) return false;
+  if (!get_encode()) return false;
   if ((ldx & 3) || (ldy & 3) || (ldw & 3)) return false;
   if ((reinterpret_cast<uintptr_t>(X) & 15) || (reinterpret_cast<uintptr_t>(dY) & 15) || (reinterpret_cast<uintptr_t>(dW) & 15)) return false;
   TnParams p;
@@ -623,10 +600,6 @@ extern "C" int magpo_test_gemm_tc(magpo_stream_t s_, int64_t M, int N, int K, co
   if (!tc_supported(M, N, K, X, ldx, Y, ldy, K)) return MAGPO_ERR_UNSUPPORTED;
   MAGPO_TRY(tc_prepare_region(s, WT, (int64_t)N * K, scratch, scratch + (int64_t)N * K));
   return gemm_tc(s, M, N, K, X, ldx, scratch, scratch + (int64_t)N * K, K, bias, Y, ldy, flags);
-}
-extern "C" int magpo_set_tensor_cores(int on) {
-  tc_set_enabled(on != 0);
-  return MAGPO_OK;
 }
 
 extern "C" int magpo_test_gemm_tc_tn(magpo_stream_t s_, int64_t M, int N, int K, const float* X, int ldx, const float* dY, int ldy,

@@ -201,10 +201,8 @@ int transposes(cudaStream_t s, const NetShape& sh, const GuiderG& p, const Ws& w
     MAGPO_TRY(transpose(s, D, 2 * D, p.dec[b].ffn_gl, w.d_glT[b]));
     MAGPO_TRY(transpose(s, D, D, p.dec[b].ffn_out, w.d_outT[b]));
   }
-  if (tc_enabled()) {
-    MAGPO_TRY(tc_prepare_region(s, w.WobsT, w.t_n, w.t_hi, w.t_lo));
-    MAGPO_TRY(tc_prepare_region(s, p.obs_scale, p.total, w.p_hi, w.p_lo));
-  }
+  MAGPO_TRY(tc_prepare_region(s, w.WobsT, w.t_n, w.t_hi, w.t_lo));
+  MAGPO_TRY(tc_prepare_region(s, p.obs_scale, p.total, w.p_hi, w.p_lo));
   return MAGPO_OK;
 }
 

@@ -162,23 +162,11 @@ __device__ __forceinline__ uint32_t idesc_tf32(int n) {  // kind::tf32, fp32 acc
   return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
 }
 
-__device__ __forceinline__ uint64_t gtimer() {
-  uint64_t t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-  return t;
-}
-// timeline probe (GRU_TIMELINE=1 tools/diag_gru.py): CTA 0 records %globaltimer at the hand-over points of the first steps
-#define GS_STAMP(role, idx)                                                                     \
-  do {                                                                                          \
-    if (p.dbg && blockIdx.x == 0 && (idx) < 1024) p.dbg[(role) * 1024 + (idx)] = gtimer();      \
-  } while (0)
-
 struct GruOutMaps {  // [T(+1), Rs, cols] tensors, boxes of [1, rpt, 32]
   CUtensorMap gi, rzn, ghn, Y, HU;
 };
 
 struct GruFwdArgs {
-  unsigned long long* dbg;
   int T, N, A;
   int64_t Rs;
   int rpt;              // rows per CTA
@@ -248,7 +236,6 @@ gru_scan_fwd_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
             for (int kc = 0; kc < 4; ++kc, ++it) {
               const int s = it % GS_FWD_STAGES;
               mbar_wait(&b_empty[s], ((it / GS_FWD_STAGES) & 1) ^ 1);
-              GS_STAMP(0, it);
               mbar_expect_tx(&b_full[s], GS_FWD_STAGE);
               uint8_t* st = sB + (size_t)s * GS_FWD_STAGE;
 #pragma unroll
@@ -266,7 +253,6 @@ gru_scan_fwd_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
         for (int t = 0; t < T; ++t) {
           mbar_wait(a_ready, t & 1);
           tc_fence_after();
-          GS_STAMP(1, t * 16);
           for (int jb = 0; jb < 4; ++jb) {
             const int acc = jb & 1;
             const uint32_t use = (uint32_t)t * 2 + (jb >> 1);  // uses of this accumulator so far
@@ -279,7 +265,6 @@ gru_scan_fwd_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
               const int s = it % GS_FWD_STAGES;
               mbar_wait(&b_full[s], (it / GS_FWD_STAGES) & 1);
               tc_fence_after();
-              if (kc == 0) GS_STAMP(1, t * 16 + 1 + jb * 2);
               const uint32_t a_hi = tmem_base + (uint32_t)(kc * 32), a_lo = a_hi + GS_F_ALO;
               const uint32_t b_hi = smem_u32(sB + (size_t)s * GS_FWD_STAGE), b_lo = b_hi + GS_FWD_STAGE / 2;
 #pragma unroll
@@ -292,7 +277,6 @@ gru_scan_fwd_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
               umma_commit(&b_empty[s]);
             }
             umma_commit(&acc_full[acc]);
-            GS_STAMP(1, t * 16 + 2 + jb * 2);
           }
         }
       }
@@ -344,10 +328,8 @@ gru_scan_fwd_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
         unstage_patch(gi_n, sIn + 2 * GS_CHUNK, 8 * cq, gg);
         __syncwarp();
         if (lane == 0) mbar_arrive(in_empty);  // the loader may fetch the next block's columns
-        if (threadIdx.x == 0) GS_STAMP(2, (t * 4 + jb) * 6 + 0);
         mbar_wait(&acc_full[jb & 1], (uint32_t)(t * 2 + (jb >> 1)) & 1u);
         tc_fence_after();
-        if (threadIdx.x == 0) GS_STAMP(2, (t * 4 + jb) * 6 + 1);
         uint32_t ar[8], az[8], an[8];
         const uint32_t tcol = tmem_lane + GS_F_ACC + (uint32_t)((jb & 1) * 96 + 8 * cq);
         tmem_ld_patch_nowait(tcol, ar);
@@ -357,7 +339,6 @@ gru_scan_fwd_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
         tc_fence_before();  // this warp's part of the accumulator is in registers: hand the buffer back
         __syncwarp();
         if (lane == 0) mbar_arrive(&acc_empty[jb & 1]);
-        if (threadIdx.x == 0) GS_STAMP(2, (t * 4 + jb) * 6 + 2);
         float y_[8];
 #pragma unroll
         for (int rr = 0; rr < 4; ++rr)
@@ -374,7 +355,6 @@ gru_scan_fwd_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
             y_[i] = hn;
             h[8 * jb + i] = keep[rr] ? hn : 0.0f;
           }
-        if (threadIdx.x == 0) GS_STAMP(2, (t * 4 + jb) * 6 + 3);
         // staging + bulk stores per group of the 4 warps that share 32 rows (sub-boxes of [32 rows x 32 floats]): the groups do not wait
         // for each other, a 128-thread barrier instead of a 512-thread one
         if (grp_live) {
@@ -400,7 +380,6 @@ gru_scan_fwd_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
             bulk_commit();
           }
         }
-        if (threadIdx.x == 0) GS_STAMP(2, (t * 4 + jb) * 6 + 4);
       }
       if (t + 1 < T) {
         // every MMA of this step has completed (the last block's acc_full was observed): the A operand may be replaced
@@ -411,7 +390,6 @@ gru_scan_fwd_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(a_ready);  // one arrival per warp: 512 serialized shared-memory arrivals cost microseconds
-        if (threadIdx.x == 0) GS_STAMP(2, (t * 4 + 3) * 6 + 5);
       }
     }
   }
@@ -669,21 +647,12 @@ gru_scan_bwd_kernel(const __grid_constant__ CUtensorMap tmWh, const __grid_const
 
 }  // namespace
 
-unsigned long long* g_gru_dbg = nullptr;
-
-// Rows per CTA. Measured on B200 (tools/gru_rpt_experiment.sh): the per-timestep chain of a scan CTA shortens when it owns fewer
+// Rows per CTA. Measured on B200 (profiles/r2_experiments.md): the per-timestep chain of a scan CTA shortens when it owns fewer
 // rows (RWARE shard, 2048 rows: 57.6 / 41.2 / 33.7 ms per step of 8 minibatches at 128 / 64 / 32 rows), but the scans run on a
 // forked stream beside the guider's persistent kernels and a scan CTA fills its SM (227 KB of shared memory): more than ~64 scan
 // CTAs starve the guider and the step gets slower (LBF, 8192 rows: GRU 63 -> 45 ms but the step 284 -> 289 ms at 64 rows). So: the
-// fewest rows per CTA that keep the scan on at most 64 SMs. MAGPO_GRU_RPT overrides, for experiments.
+// fewest rows per CTA that keep the scan on at most 64 SMs.
 static int gru_rows_per_tile(int64_t Rs) {
-  static int forced = -1;
-  if (forced < 0) {
-    const char* e = getenv("MAGPO_GRU_RPT");
-    const int v = e ? atoi(e) : 0;
-    forced = (v >= 8 && v <= 128) ? v : 0;
-  }
-  if (forced) return forced;
   if (ceil_div(Rs, 32) <= 64) return 32;
   if (ceil_div(Rs, 64) <= 64) return 64;
   return 128;
@@ -703,7 +672,7 @@ int gru_scan_fwd(cudaStream_t s, int T, int N, int A, const float* gi, const flo
   if (!tc_make_map3(&om.gi, gi, T, Rs, 3 * kH, rpt) || !tc_make_map3(&om.rzn, rzn, T, Rs, 3 * kH, ob) || !tc_make_map3(&om.ghn, ghn, T, Rs, kH, ob) ||
       !tc_make_map3(&om.Y, Y, T, Rs, kH, ob) || !tc_make_map3(&om.HU, HU, T + 1, Rs, kH, ob))
     return MAGPO_ERR_ARG;
-  GruFwdArgs a{g_gru_dbg, T, N, A, Rs, rpt, gi, bhn, done, rzn, ghn, Y, HU};
+  GruFwdArgs a{T, N, A, Rs, rpt, gi, bhn, done, rzn, ghn, Y, HU};
   // per row and step: 3xTF32 MMAs are the pipe work; bytes: gi 1536 read, rzn+ghn+Y+HU 3072 written
   ProfScope ps(PROF_GRU, s, 4608.0 * (double)Rs * T);
   gru_scan_fwd_kernel<<<(unsigned)ceil_div(Rs, rpt), GS_THREADS, GS_SMEM, s>>>(tmh, tml, om, a);
@@ -732,12 +701,6 @@ int gru_scan_bwd(cudaStream_t s, int T, int N, int A, const float* dY, const flo
 }
 
 }  // namespace magpo
-
-// GRU_TIMELINE=1 tools/diag_gru.py: device buffer of 3 x 1024 uint64 %globaltimer stamps written by CTA 0 of the forward scan
-extern "C" int magpo_debug_gru_timeline(unsigned long long* buf) {
-  magpo::g_gru_dbg = buf;
-  return MAGPO_OK;
-}
 
 // Host-only: the rows per CTA both scans launch with for Rs = N * A rows (tests assert which tile branch a case covers).
 extern "C" int magpo_debug_gru_rows_per_tile(int64_t Rs) { return magpo::gru_rows_per_tile(Rs); }

@@ -27,8 +27,6 @@ inline Wref wref(const float* w, int ldw, const float* wt = nullptr, int ldwt = 
 int gemm_nn(cudaStream_t s, int64_t M, int N, int K, const float* X, int ldx, Wref W, const float* bias, float* Y,
             int ldy, int flags);
 // ---- gemm_tc.cu (tcgen05 + TMA, 3xTF32)
-void tc_set_enabled(bool on);
-bool tc_enabled();
 int tc_prepare_region(cudaStream_t s, const float* base, int64_t n, float* hi, float* lo);
 bool tc_lookup(const float* w, const float** hi, const float** lo);
 bool tc_supported(int64_t M, int N, int K, const float* X, int ldx, const float* Y, int ldy, int ldb);

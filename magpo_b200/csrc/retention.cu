@@ -250,15 +250,13 @@ int retention_chunk_bwd(cudaStream_t s, int T, int N, int A, float kappa, bool c
                         const float* v, int ld, const uint8_t* done, const float* Hck, const float* dret, float* dq,
                         float* dk, float* dv, int ldd);
 
-static bool g_force_scan = false;  // tools/bench_retention.py: A/B against the register scan
-
 int retention_fwd(cudaStream_t s, int T, int N, int A, float kappa, bool causal, const float* q, const float* k,
                   const float* v, int ld, const float* H0, const uint8_t* done, float* ret, float* Hsave,
                   float* Hout) {
   if (T <= 0 || N <= 0) return MAGPO_OK;
   if (A < 1 || A > kMaxAgents || (ld & 3)) return MAGPO_ERR_UNSUPPORTED;
   // sequences (the update) run chunkwise on the tensor cores; a single step (the rollout) keeps the register scan
-  if (T > 1 && !g_force_scan) return retention_chunk_fwd(s, T, N, A, kappa, causal, q, k, v, ld, H0, done, ret, Hsave, Hout);
+  if (T > 1) return retention_chunk_fwd(s, T, N, A, kappa, causal, q, k, v, ld, H0, done, ret, Hsave, Hout);
   const size_t smem = (size_t)(3 * A * 64 + A * 16 * 64) * sizeof(float);
   ProfScope ps(PROF_RET_FWD, s, 4.0 * 4096.0 * (double)T * N * A);
   if (causal) {
@@ -278,7 +276,7 @@ int retention_bwd(cudaStream_t s, int T, int N, int A, float kappa, bool causal,
   (void)H0;
   if (T <= 0 || N <= 0) return MAGPO_OK;
   if (A < 1 || A > kMaxAgents || (ld & 3) || (ldd & 3)) return MAGPO_ERR_UNSUPPORTED;
-  if (T > 1 && !g_force_scan) return retention_chunk_bwd(s, T, N, A, kappa, causal, q, k, v, ld, done, Hsave, dret, dq, dk, dv, ldd);
+  if (T > 1) return retention_chunk_bwd(s, T, N, A, kappa, causal, q, k, v, ld, done, Hsave, dret, dq, dk, dv, ldd);
   const size_t smem = (size_t)(4 * A * 64 + A * 16 * 64) * sizeof(float);
   ProfScope ps(PROF_RET_BWD, s, 10.0 * 4096.0 * (double)T * N * A);
   if (causal) {
@@ -295,11 +293,6 @@ int retention_bwd(cudaStream_t s, int T, int N, int A, float kappa, bool causal,
 }  // namespace magpo
 
 using namespace magpo;
-
-extern "C" int magpo_debug_force_retention_scan(int on) {
-  magpo::g_force_scan = on != 0;
-  return MAGPO_OK;
-}
 
 // Test hook: retention forward/backward on caller buffers (q,k,v packed with row stride ld).
 extern "C" int magpo_test_retention(magpo_stream_t s, int bwd, int T, int N, int A, float kappa, int causal,

@@ -35,8 +35,6 @@ int sable_step(cudaStream_t st, const MagpoNetCfg* net, int B, int gumbel_rows, 
 
 namespace {
 
-bool g_force_unfused = false;  // tests / tools: A/B the fused step kernel against the per-layer launch sequence
-
 // keys: [T+1][A][2] sample keys; key advanced in place by T+1 splits.
 __global__ void rollout_keys_kernel(uint32_t* __restrict__ key, int steps, int A, uint32_t* __restrict__ sample_keys) {
   if (blockIdx.x != 0 || threadIdx.x != 0) return;
@@ -118,19 +116,6 @@ __global__ void copy_zero_done_kernel(int64_t B, int64_t quads /* float4 per env
 
 inline unsigned g256(int64_t n) { return (unsigned)ceil_div(n, 256); }
 
-// The learner's GRU push (rec_magpo.py:146-159) needs only the observations, not the guider's actions, and nothing reads the learner's
-// hidden state before the rollout ends: instead of 5 small launches per env step it can run once per `chunk` env steps as one batched
-// pre-torso + input projection and one persistent GRU scan over the chunk's timesteps (MAGPO_ROLLOUT_LEARNER_CHUNK; default 1 = per step).
-inline int learner_chunk_steps() {
-  static int c = -1;
-  if (c < 0) {
-    const char* e = getenv("MAGPO_ROLLOUT_LEARNER_CHUNK");
-    c = e ? atoi(e) : 1;
-    if (c < 1) c = 1;
-  }
-  return c;
-}
-
 struct RolloutWs {
   SableActs sa;
   ActorActs aa;
@@ -141,24 +126,10 @@ struct RolloutWs {
   uint32_t* sample_keys;
   void* gws;  // general guider shapes (generic.cuh): the step workspace of sable_g_get_actions instead of the default path's buffers
   size_t gws_bytes;
-  ActorActs ac;  // the learner's state push in chunks of `chunk` env steps (persistent GRU scan instead of per-step launches)
-  int chunk;
   void plan(Arena& ar, const MagpoNetCfg* net, int B, int T) {
     const int64_t R = (int64_t)B * net->n_agents;
     aa.plan(ar, R, R, net->action_dim, false);
     at.plan(ar, net->action_dim);
-    chunk = std::min(T, learner_chunk_steps());
-    ac = ActorActs{};
-    if (chunk > 1) {
-      const size_t rH = (size_t)chunk * R * kH;
-      ac.e = ar.get<float>(rH);
-      ac.gi = ar.get<float>(3 * rH);
-      ac.gh = ar.get<float>((size_t)R * 3 * kH);
-      ac.HU = ar.get<float>(rH + (size_t)R * kH);
-      ac.Y = ar.get<float>(rH);
-      ac.rzn = ar.get<float>(3 * rH);
-      ac.ghn = ar.get<float>(rH);
-    }
     sample_keys = ar.get<uint32_t>((size_t)(T + 1) * net->n_agents * 2);
     gws = nullptr; gws_bytes = 0;
     const NetShape shape = NetShape::of(net);
@@ -190,7 +161,7 @@ int get_actions(cudaStream_t s, const MagpoNetCfg* net, int B, int gumbel_rows, 
   if (w.gws)  // general (embed_dim, n_head, n_block): layer by layer (the caller prepared the workspace once: sable_g_prepare)
     return sable_g_get_actions(s, net, B, gumbel_rows, gp.obs_scale, agents_view, action_mask, step_count, prev_done, sample_keys, hs, dry,
                                action, log_prob, value, masked_logits, w.gws, w.gws_bytes, false);
-  if (!g_force_unfused && sable_step_supported(A, d, a))
+  if (sable_step_supported(A, d, a))
     return sable_step(s, net, B, gumbel_rows, gp, kappa, agents_view, action_mask, step_count, prev_done, sample_keys, w.pe, w.dec_tab,
                       hs, dry, action, log_prob, value, masked_logits);
   MAGPO_TRY(sable_encoder_forward(s, gp, gt, 1, B, A, d, ms, agents_view, step_count, prev_done, hs.encoder, kappa, w.pe,
@@ -235,11 +206,6 @@ using namespace magpo;
 
 extern "C" {
 
-int magpo_debug_force_unfused_rollout(int on) {
-  g_force_unfused = on != 0;
-  return MAGPO_OK;
-}
-
 size_t magpo_rollout_workspace_bytes(const MagpoNetCfg* net, int32_t B, int32_t T) {
   if (check_net(net) != MAGPO_OK || B < 0 || T < 0) return 0;
   Arena ar(nullptr, SIZE_MAX);
@@ -266,7 +232,7 @@ int magpo_sable_get_actions(MagpoContext* ctx_, magpo_stream_t s_, const MagpoNe
     return sable_g_get_actions(s, net, B, gumbel_rows, guider, agents_view, action_mask, step_count, prev_done, sample_keys, hs, false, action,
                                log_prob, value, logits, w.gws, w.gws_bytes, true);
   MAGPO_TRY(build_pe_table(s, net->max_step_count, w.pe, net->timestep_pe != 0));
-  if (!g_force_unfused && sable_step_supported(net->n_agents, net->obs_dim, net->action_dim))
+  if (sable_step_supported(net->n_agents, net->obs_dim, net->action_dim))
     MAGPO_TRY(sable_step_tables(s, net, GuiderP::bind(const_cast<float*>(guider), net->obs_dim, net->action_dim), w.pe, w.dec_tab));
   const GuiderP gp = GuiderP::bind(const_cast<float*>(guider), net->obs_dim, net->action_dim);
   return get_actions(s, net, B, gumbel_rows, gp, nullptr, net_kappa(net), agents_view, action_mask, step_count, prev_done,
@@ -314,20 +280,17 @@ int magpo_rollout(MagpoContext* ctx_, magpo_stream_t s_, const MagpoNetCfg* net,
   if (w.gws) {  // general guider shape: PE table, transposed weights and their TF32 images once per rollout
     gp.obs_scale = const_cast<float*>(guider);  // get_actions hands the flat buffer to the general path
     MAGPO_TRY(sable_g_prepare(s, net, B, guider, w.gws, w.gws_bytes));
-    if (tc_enabled()) {
-      MAGPO_TRY(actor_transpose(s, ap, w.at, a));
-      atp = &w.at;
-    }
+    MAGPO_TRY(actor_transpose(s, ap, w.at, a));
+    atp = &w.at;
   } else {
     MAGPO_TRY(build_pe_table(s, net->max_step_count, w.pe, net->timestep_pe != 0));
-    if (!g_force_unfused && sable_step_supported(net->n_agents, net->obs_dim, net->action_dim))
+    if (sable_step_supported(net->n_agents, net->obs_dim, net->action_dim))
       MAGPO_TRY(sable_step_tables(s, net, GuiderP::bind(const_cast<float*>(guider), net->obs_dim, net->action_dim), w.pe, w.dec_tab));
-    if (tc_enabled()) {  // parameters are constant during the rollout: one transpose + TF32 split up front
-      MAGPO_TRY(guider_transpose(s, gp, w.gt, d));
-      MAGPO_TRY(actor_transpose(s, ap, w.at, a));
-      gtp = &w.gt;
-      atp = &w.at;
-    }
+    // parameters are constant during the rollout: one transpose + TF32 split up front
+    MAGPO_TRY(guider_transpose(s, gp, w.gt, d));
+    MAGPO_TRY(actor_transpose(s, ap, w.at, a));
+    gtp = &w.gt;
+    atp = &w.at;
   }
   if (carry_over) {  // LearnerState.timestep of the previous call becomes observation slot 0
     MAGPO_CUDA_OK(cudaMemcpyAsync(traj.done, traj.done + (size_t)T * B, B, cudaMemcpyDeviceToDevice, s));
@@ -363,19 +326,11 @@ int magpo_rollout(MagpoContext* ctx_, magpo_stream_t s_, const MagpoNetCfg* net,
     const int32_t* stepc = traj.step_count + (size_t)t * BA;
     const uint8_t* prev_done = traj.done + (size_t)t * B;
     int32_t* act = traj.action + (size_t)t * BA;
-    const bool chunked = w.chunk > 1 && atp && !sys->sable_only;
-    const bool push_now = !chunked || (t + 1) % w.chunk == 0 || t == T - 1;
-    if (overlap && push_now) {  // observation slot t and done[t] are complete on `s` here
+    if (overlap) {  // observation slot t and done[t] are complete on `s` here
       MAGPO_CUDA_OK(cudaEventRecord(g_rside.fork, s));
       MAGPO_CUDA_OK(cudaStreamWaitEvent(s2, g_rside.fork, 0));
     }
-    if (chunked && push_now) {
-      const int t0 = (t / w.chunk) * w.chunk, len = t - t0 + 1;
-      MAGPO_TRY(actor_forward(s2, ap, atp, len, B, A, d, a, traj.agents_view + (size_t)t0 * BA * d, traj.done + (size_t)t0 * B, policy_h, w.ac,
-                              nullptr, policy_h));
-    } else if (!chunked && !sys->sable_only) {
-      MAGPO_TRY(actor_forward(s2, ap, atp, 1, B, A, d, a, obs, prev_done, policy_h, w.aa, nullptr, policy_h));
-    }
+    if (!sys->sable_only) MAGPO_TRY(actor_forward(s2, ap, atp, 1, B, A, d, a, obs, prev_done, policy_h, w.aa, nullptr, policy_h));
     MAGPO_TRY(get_actions(s, net, B, E, gp, gtp, kappa, obs, mask, stepc, prev_done, w.sample_keys + (size_t)t * A * 2, hs,
                           false, act, traj.log_prob + (size_t)t * BA, traj.value + (size_t)t * BA, nullptr, w));
     MagpoTimeStep o = ts;

@@ -43,7 +43,7 @@ int guider_transpose(cudaStream_t s, const GuiderP& p, const GuiderT& t, int d) 
   MAGPO_TRY(transpose(s, kD, 2 * kD, p.dffn_gl, t.dffn_glT));
   MAGPO_TRY(transpose(s, kD, kD, p.dffn_out, t.dffn_outT));
   MAGPO_TRY(transpose(s, kD, kD, p.dh0_w, t.dh0T));
-  if (tc_enabled()) MAGPO_TRY(tc_prepare_region(s, t.WobsT, t.region_n, t.region_hi, t.region_lo));
+  MAGPO_TRY(tc_prepare_region(s, t.WobsT, t.region_n, t.region_hi, t.region_lo));
   return MAGPO_OK;
 }
 
@@ -183,12 +183,7 @@ int sable_decoder_forward(cudaStream_t s, const GuiderP& p, const GuiderT* pt, i
 // at 0.3-0.7 of the HBM roofline each, so together they use the memory system better than one after the other.
 int sable_train_forward(cudaStream_t s, const GuiderP& p, const GuiderT* pt, const SableBatch& b, const SableActs& w,
                         float* value, float* logits, bool save_states) {
-  static int split = -1;
-  if (split < 0) {
-    const char* e = getenv("MAGPO_DEC_OVERLAP");
-    split = e ? atoi(e) : 1;
-  }
-  const bool overlap = split && nets_overlap_enabled();
+  const bool overlap = nets_overlap_enabled();
   float* hs_self = save_states ? w.Hs_self : nullptr;
   float* hs_cross = save_states ? w.Hs_cross : nullptr;
   ForkJoin& g_dec = ctx().dec;

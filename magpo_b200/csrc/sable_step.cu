@@ -39,7 +39,6 @@ constexpr unsigned kFull = 0xffffffffu;
 
 struct StepArgs {
   int B, d, a, max_step, gumbel_rows, dry;
-  int keep_l2;               // decoder-state reads before the last agent's pass keep the default L2 policy (MAGPO_STEP_KEEP_L2, default 1)
   float kappa;
   const float* obs;          // [B,A,d]
   const uint8_t* mask;       // [B,A,a]
@@ -152,7 +151,7 @@ __device__ __forceinline__ void prefetch_state(const float* H) {
 
 // state rows r0..r0+7 of env state H. KEEP = false: evict-first (the last read of the state in this launch). KEEP = true: default
 // policy — a decoder state is read once per agent, and next to evict-first streams the lines of an earlier agent's pass survive in
-// L2 longer (tools/step_l2_experiment.sh: RWARE shard, 1024 envs x 4 agents, whose states fit L2: rollout 23.3 -> 22.3 ms in both
+// L2 longer (profiles/r2_experiments.md: RWARE shard, 1024 envs x 4 agents, whose states fit L2: rollout 23.3 -> 22.3 ms in both
 // A/B runs; LBF, 8192 envs x 2 agents: 49.8 -> 48.4 ms in one A/B run and no difference in two others, DRAM bytes per launch
 // unchanged under ncu; explicit evict_last / evict_normal createpolicy operands and a second L2 prefetch between the passes
 // measured no better)
@@ -176,7 +175,7 @@ __device__ __forceinline__ void load_rows(float2 (&h)[8], const float* __restric
 template <int A, int EPW>
 __device__ __forceinline__ void decoder_retention(int i, float* __restrict__ Hall, const int (&b)[EPW], const bool (&live)[EPW],
                                                   const float (&lam)[EPW], const float2 (&q)[EPW], const float2 (&k)[EPW][A],
-                                                  const float2 (&v)[EPW][A], float2 (&out)[EPW], int lane, bool keep_l2) {
+                                                  const float2 (&v)[EPW][A], float2 (&out)[EPW], int lane) {
   float2 acc[EPW];
 #pragma unroll
   for (int e = 0; e < EPW; ++e) acc[e] = make_float2(0.f, 0.f);
@@ -184,7 +183,7 @@ __device__ __forceinline__ void decoder_retention(int i, float* __restrict__ Hal
     float2 h[EPW][8];
 #pragma unroll
     for (int e = 0; e < EPW; ++e) {
-      if (i == A - 1 || !keep_l2) load_rows<false>(h[e], Hall + (size_t)b[e] * kD * kD, r0, lane);
+      if (i == A - 1) load_rows<false>(h[e], Hall + (size_t)b[e] * kD * kD, r0, lane);
       else load_rows<true>(h[e], Hall + (size_t)b[e] * kD * kD, r0, lane);
     }
 #pragma unroll
@@ -474,7 +473,7 @@ sable_step_kernel(const GuiderP p, const StepArgs s) {
       float2 q1[EPW];
 #pragma unroll
       for (int e = 0; e < EPW; ++e) q1[e] = qkvg[e][0];
-      decoder_retention<A, EPW>(i, s.h_self, b, live, lam, q1, k1, v1, r1, lane, s.keep_l2 != 0);
+      decoder_retention<A, EPW>(i, s.h_self, b, live, lam, q1, k1, v1, r1, lane);
     }
     float2 rpe[EPW];
     {
@@ -524,7 +523,7 @@ sable_step_kernel(const GuiderP p, const StepArgs s) {
         for (int jj = 0; jj < A; ++jj)
           if (jj == i) { k2[e][jj] = kvg[e][0]; v2[e][jj] = kvg[e][1]; }
       }
-      decoder_retention<A, EPW>(i, s.h_cross, b, live, lam, q2, k2, v2, r2, lane, s.keep_l2 != 0);
+      decoder_retention<A, EPW>(i, s.h_cross, b, live, lam, q2, k2, v2, r2, lane);
       const float2 gs = ldg2(p.gn2_s + 2 * lane), gb = ldg2(p.gn2_b + 2 * lane), dln2 = ldg2(p.dln2 + 2 * lane);
       float2 t[EPW], o[EPW];
 #pragma unroll
@@ -633,14 +632,8 @@ decoder_tables_kernel(const GuiderP p, int a, int max_step, const float* __restr
 
 // Warps per CTA. Two CTAs share an SM (296 CTA slots): pick the CTA size whose last wave is fullest; small batches keep >= 6 warps,
 // because every CTA streams the step's weights (0.4 MB) through its own shared memory (RWARE shard of 1024 envs, rollout of 128
-// steps: 118 ms at 4 warps per CTA, 34.8 ms at 7 — tools/step_warps_experiment.sh).
+// steps: 118 ms at 4 warps per CTA, 34.8 ms at 7 — profiles/r2_experiments.md).
 int pick_warps(int64_t units) {
-  static int forced_warps = -1;
-  if (forced_warps < 0) {
-    const char* e = getenv("MAGPO_STEP_WARPS");
-    forced_warps = e ? std::min(std::max(atoi(e), 1), SS_WARPS) : 0;
-  }
-  if (forced_warps) return forced_warps;
   const int64_t slots = 2 * kNumSMs;
   int best = 7;
   double best_eff = -1.0;
@@ -675,14 +668,7 @@ int launch_ae(cudaStream_t st, const GuiderP& p, const StepArgs& s) {
 }
 
 // envs per warp: 2 when the batch fills the 296 CTA slots anyway, 1 below that (twice the warps, half the chain per warp)
-int envs_per_warp(int64_t B) {
-  static int forced_epw = -1;
-  if (forced_epw < 0) {
-    const char* e = getenv("MAGPO_STEP_EPW");
-    forced_epw = e ? atoi(e) : 0;
-  }
-  return (forced_epw == 1 || forced_epw == 2) ? forced_epw : (B <= 2048 ? 1 : 2);
-}
+int envs_per_warp(int64_t B) { return B <= 2048 ? 1 : 2; }
 
 template <int A>
 int launch_a(cudaStream_t st, const GuiderP& p, const StepArgs& s) {
@@ -713,12 +699,6 @@ int sable_step(cudaStream_t st, const MagpoNetCfg* net, int B, int gumbel_rows, 
   StepArgs s;
   s.B = B; s.d = net->obs_dim; s.a = net->action_dim; s.max_step = net->max_step_count; s.gumbel_rows = gumbel_rows;
   s.dry = (dry || !action) ? 1 : 0;
-  static int keep_l2 = -1;
-  if (keep_l2 < 0) {
-    const char* e = getenv("MAGPO_STEP_KEEP_L2");
-    keep_l2 = e ? (atoi(e) != 0) : 1;
-  }
-  s.keep_l2 = keep_l2;
   s.kappa = kappa;
   s.obs = agents_view; s.mask = action_mask; s.step = step_count; s.prev_done = prev_done; s.keys = sample_keys; s.pe = pe;
   s.dec_tab = dec_tab;

@@ -191,8 +191,6 @@ SableBatch make_batch(const MagpoNetCfg* net, const MagpoMinibatch& mb, const fl
   return b;
 }
 
-int g_debug_skip = 0;  // tools/bench_phases.py only: bit0 guider fwd+bwd, bit1 learner fwd+bwd, bit2 guider bwd, bit3 learner bwd
-
 int check_mb(const MagpoMinibatch& mb) {
   if (mb.T < 1 || mb.N < 1 || !mb.agents_view || !mb.action_mask || !mb.step_count || !mb.done || !mb.action ||
       !mb.sable_h0.encoder || !mb.sable_h0.decoder_self || !mb.sable_h0.decoder_cross)
@@ -321,14 +319,11 @@ int magpo_minibatch_grads(MagpoContext* ctx_, magpo_stream_t s_, const MagpoNetC
     MAGPO_TRY(build_pe_table(s, net->max_step_count, w.pe, net->timestep_pe != 0));
     MAGPO_TRY(guider_transpose(s, gp, w.gt, d));
   }
-  if (tc_enabled()) {
-    if (!general) MAGPO_TRY(tc_prepare_region(s, guider, gp.total, w.g_hi, w.g_lo));
-    MAGPO_TRY(tc_prepare_region(s, actor, ap.total, w.a_hi, w.a_lo));
-  }
+  if (!general) MAGPO_TRY(tc_prepare_region(s, guider, gp.total, w.g_hi, w.g_lo));
+  MAGPO_TRY(tc_prepare_region(s, actor, ap.total, w.a_hi, w.a_lo));
   const SableBatch b = make_batch(net, mb, w.pe);
-  const int skip = g_debug_skip;
-  bool skip_learner = false;
-  const bool overlap = g_overlap_nets && !skip && !sys->sable_only;
+  const bool sable_only = sys->sable_only != 0;
+  const bool overlap = g_overlap_nets && !sable_only;
   cudaStream_t s2 = s, sg = s;  // learner stream, guider stream
   ForkJoin& g_side = ctx().side;
   if (overlap) {
@@ -336,17 +331,13 @@ int magpo_minibatch_grads(MagpoContext* ctx_, magpo_stream_t s_, const MagpoNetC
     MAGPO_CUDA_OK(cudaEventRecord(g_side.fork, s));
     MAGPO_CUDA_OK(cudaStreamWaitEvent(g_side.s, g_side.fork, 0));
   }
-  const bool sable_only = sys->sable_only != 0;
-  if (sable_only) skip_learner = true;
-  if (!(skip & 2) && !skip_learner)
+  if (!sable_only)
     MAGPO_TRY(actor_forward(s2, ap, &w.at, T, N, A, d, a, mb.agents_view, mb.done, mb.policy_h0, w.aa, w.ll, nullptr));
-  if (!(skip & 1)) {
-    if (general)
-      MAGPO_TRY(sable_g_train_forward(sg, net, guider, T, N, mb.agents_view, mb.step_count, mb.done, mb.action, mb.sable_h0.encoder,
-                                      mb.sable_h0.decoder_self, mb.sable_h0.decoder_cross, w.value, w.lg, w.gws, w.gws_bytes, true));
-    else
-      MAGPO_TRY(sable_train_forward(sg, gp, &w.gt, b, w.sa, w.value, w.lg, true));
-  }
+  if (general)
+    MAGPO_TRY(sable_g_train_forward(sg, net, guider, T, N, mb.agents_view, mb.step_count, mb.done, mb.action, mb.sable_h0.encoder,
+                                    mb.sable_h0.decoder_self, mb.sable_h0.decoder_cross, w.value, w.lg, w.gws, w.gws_bytes, true));
+  else
+    MAGPO_TRY(sable_train_forward(sg, gp, &w.gt, b, w.sa, w.value, w.lg, true));
   if (overlap) {
     MAGPO_CUDA_OK(cudaEventRecord(g_side.join, g_side.s));
     MAGPO_CUDA_OK(cudaStreamWaitEvent(s, g_side.join, 0));
@@ -360,30 +351,22 @@ int magpo_minibatch_grads(MagpoContext* ctx_, magpo_stream_t s_, const MagpoNetC
     MAGPO_CUDA_OK(cudaEventRecord(g_side.fork, s));
     MAGPO_CUDA_OK(cudaStreamWaitEvent(g_side.s, g_side.fork, 0));
   }
-  if (!(skip & 10) && !skip_learner) MAGPO_TRY(actor_backward(s2, ap, w.at, T, N, A, d, a, mb.agents_view, mb.done, w.aa, w.dll, ag));
+  if (!sable_only) MAGPO_TRY(actor_backward(s2, ap, w.at, T, N, A, d, a, mb.agents_view, mb.done, w.aa, w.dll, ag));
   // pmean over "device" (rec_magpo.py:399-409), issued where the gradients are produced: the learner's half (+ the 8 loss sums, which
   // lie behind it) as soon as the learner's backward is done — on its own stream, under the guider's remaining backward — and the
   // guider's half at the end. Every rank issues the two all-reduces in this order.
   MagpoComm* comm = reduce_grads ? ctx().comm : nullptr;
-  static int comm_split = -1;
-  if (comm_split < 0) {
-    const char* e = getenv("MAGPO_COMM_SPLIT");  // experiments: "0" = one all-reduce of the whole buffer after the guider's backward
-    comm_split = !(e && e[0] == '0');
-  }
-  if (comm && comm_split) MAGPO_TRY(comm_allreduce(comm, s2, grads + gp.total, ap.total + 8, 0));
-  if (!(skip & 5)) {
-    if (general)
-      MAGPO_TRY(sable_g_train_backward(sg, net, guider, T, N, mb.agents_view, mb.step_count, mb.done, mb.action, mb.sable_h0.encoder,
-                                       mb.sable_h0.decoder_self, mb.sable_h0.decoder_cross, w.dlg, w.dvalue, grads, w.gws, w.gws_bytes));
-    else
-      MAGPO_TRY(sable_train_backward(sg, gp, w.gt, b, w.sa, w.dlg, w.dvalue, gg));
-  }
-  if (comm && comm_split) MAGPO_TRY(comm_allreduce(comm, sg, grads, gp.total, 0));
+  if (comm) MAGPO_TRY(comm_allreduce(comm, s2, grads + gp.total, ap.total + 8, 0));
+  if (general)
+    MAGPO_TRY(sable_g_train_backward(sg, net, guider, T, N, mb.agents_view, mb.step_count, mb.done, mb.action, mb.sable_h0.encoder,
+                                     mb.sable_h0.decoder_self, mb.sable_h0.decoder_cross, w.dlg, w.dvalue, grads, w.gws, w.gws_bytes));
+  else
+    MAGPO_TRY(sable_train_backward(sg, gp, w.gt, b, w.sa, w.dlg, w.dvalue, gg));
+  if (comm) MAGPO_TRY(comm_allreduce(comm, sg, grads, gp.total, 0));
   if (overlap) {
     MAGPO_CUDA_OK(cudaEventRecord(g_side.join, g_side.s));
     MAGPO_CUDA_OK(cudaStreamWaitEvent(s, g_side.join, 0));
   }
-  if (comm && !comm_split) MAGPO_TRY(comm_allreduce(comm, s, grads, gp.total + ap.total + 8, 0));
   return MAGPO_OK;
 }
 
@@ -430,12 +413,6 @@ int magpo_actor_forward(MagpoContext* ctx_, magpo_stream_t s_, const MagpoNetCfg
   const int64_t n = (int64_t)mb.T * mb.N * net->n_agents * net->action_dim;
   mask_logits_kernel<<<(unsigned)ceil_div(n, 256), 256, 0, s>>>(n, mb.action_mask, logits);
   MAGPO_LAUNCH_OK();
-  return MAGPO_OK;
-}
-
-// Timing hook for tools/bench_phases.py (never set by the product path): skip parts of magpo_minibatch_grads.
-int magpo_debug_set_skip(int mask) {
-  g_debug_skip = mask;
   return MAGPO_OK;
 }
 

@@ -131,7 +131,7 @@ def test_guider_and_actor_forward(dev, A, d, a, T, N):
 
 # The (3,4,10,9,50,2) case is ill-conditioned: one of its tokens has a nearly constant retention output, so the GroupNorm
 # that follows (flax "fast variance", 1/sigma large) amplifies fp32 rounding ~1000x. The plain-fp32 SIMT path measures 6e-4
-# against the fp64 oracle there (tools/diag_grads.py), so that case is held to 2e-3; well-conditioned cases sit at ~5e-6.
+# against the fp64 oracle there (profiles/r2_experiments.md), so that case is held to 2e-3; well-conditioned cases sit at ~5e-6.
 @pytest.mark.parametrize("A,d,a,T,Ns,U,tol", [(3, 4, 10, 12, 5, 2, 2e-4), (4, 75, 5, 6, 3, 1, 2e-4), (3, 4, 10, 9, 50, 2, 2e-3),
                                               (3, 4, 10, 9, 100, 2, 2e-4), (2, 14, 6, 7, 40, 1, 2e-4)])
 def test_minibatch_grads(dev, A, d, a, T, Ns, U, tol, shape=(64, 1, 1), yardstick=False):

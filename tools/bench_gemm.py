@@ -58,12 +58,7 @@ for (K, N) in [(64, 64), (64, 128), (64, 256), (128, 128), (128, 384)]:
     dY = torch.randn(M, N, device=dev)
     dW = torch.zeros(K, N, device=dev)
     ms_tc = timeit(lambda: L.call("magpo_test_gemm_tc_tn", s, C.c_int64(M), N, K, L.ptr(X), K, L.ptr(dY), N, L.ptr(dW), N))
-    os.environ["X"] = "1"
-    L.lib().magpo_set_tensor_cores(0)
-    ms_simt = timeit(lambda: L.call("magpo_test_gemm", s, 1, C.c_int64(M), N, K, L.ptr(X), L.ptr(dY), None, L.ptr(dW), 0))
-    L.lib().magpo_set_tensor_cores(1)
     gb = M * (K + N) * 4 / 1e9
     tf = 2.0 * M * N * K / 1e12
-    print(f"TN K={K:3d} N={N:3d}: tcgen05 {ms_tc:7.3f} ms  {gb / ms_tc * 1e3:7.0f} GB/s ({gb / ms_tc * 1e3 / peak:4.2f} of HBM)  {tf / ms_tc * 1e3:6.1f} TF/s"
-          f" | SIMT {ms_simt:7.3f} ms {tf / ms_simt * 1e3:6.1f} TF/s")
+    print(f"TN K={K:3d} N={N:3d}: tcgen05 {ms_tc:7.3f} ms  {gb / ms_tc * 1e3:7.0f} GB/s ({gb / ms_tc * 1e3 / peak:4.2f} of HBM)  {tf / ms_tc * 1e3:6.1f} TF/s")
     del X, dY

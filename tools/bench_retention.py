@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Micro-benchmark of the retention kernels (chunkwise tensor-core vs. register scan) at the update's shape."""
+"""Micro-benchmark of the chunkwise tensor-core retention kernels at the update's shape."""
 import argparse
 import ctypes as C
 import os
@@ -15,7 +15,6 @@ ap.add_argument("--T", type=int, default=128)
 ap.add_argument("--N", type=int, default=4096)
 ap.add_argument("--A", type=int, default=3)
 ap.add_argument("--reps", type=int, default=3)
-ap.add_argument("--only-chunk", action="store_true")
 args = ap.parse_args()
 T, N, A = args.T, args.N, args.A
 dev = torch.device("cuda:0")
@@ -30,7 +29,6 @@ Hout = torch.zeros(N, 64, 64, device=dev)
 done = (torch.rand(T, N, device=dev) < 0.01).to(torch.uint8)
 s = L.stream_ptr()
 base, db = pk.data_ptr(), dpk.data_ptr()
-lib = L.lib()
 tokens = T * N * A
 
 
@@ -57,13 +55,10 @@ def timeit(fn):
 
 
 print(f"T={T} N={N} A={A} tokens={tokens}")
-for mode in ((0,) if args.only_chunk else (0, 1)):
-    lib.magpo_debug_force_retention_scan(mode)
-    for causal in (0, 1):
-        run(0, causal)  # the backward reads the states of the matching forward
-        f = timeit(lambda: run(0, causal))
-        b = timeit(lambda: run(1, causal))
-        fb, bb = tokens * 4 * 256, tokens * 7 * 256
-        print(f"{'scan ' if mode else 'chunk'} causal={causal}: fwd {f:7.3f} ms ({fb / f / 1e6:7.0f} GB/s algorithmic)   "
-              f"bwd {b:7.3f} ms ({bb / b / 1e6:7.0f} GB/s algorithmic)")
-lib.magpo_debug_force_retention_scan(0)
+for causal in (0, 1):
+    run(0, causal)  # the backward reads the states of the matching forward
+    f = timeit(lambda: run(0, causal))
+    b = timeit(lambda: run(1, causal))
+    fb, bb = tokens * 4 * 256, tokens * 7 * 256
+    print(f"chunk causal={causal}: fwd {f:7.3f} ms ({fb / f / 1e6:7.0f} GB/s algorithmic)   "
+          f"bwd {b:7.3f} ms ({bb / b / 1e6:7.0f} GB/s algorithmic)")

@@ -1,4 +1,4 @@
-"""Diagnostic: one update step (E=8,U=2,T=16,P=2,M=2) CUDA vs oracle, tensor cores on and off.
+"""Diagnostic: one update step (E=8,U=2,T=16,P=2,M=2) CUDA vs oracle.
 Prints the six losses per (epoch, minibatch) and, per parameter tensor, |cuda - oracle| / |update|."""
 import os
 import sys
@@ -10,14 +10,12 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np
 import torch
 
-from magpo_b200 import _lib as L
 from magpo_b200.learner import MagpoLearner
 from oracle import learner as olr
 from test_gpu_learner import build
 
 
-def run(tc: int, chunk: int):
-    L.lib().magpo_set_tensor_cores(tc)
+def run(chunk: int):
     spec, ncfg, osys, state, lrn = build(torch.device("cuda:0"), E=8, U=2, T=16, P=2, M=2, chunk=chunk)
     g0 = {k: v.copy() for k, v in state["guider_params"].items()}
     a0 = {k: v.copy() for k, v in state["actor_params"].items()}
@@ -26,7 +24,7 @@ def run(tc: int, chunk: int):
     _, losses = lrn.update_step()
     torch.cuda.synchronize()
     li = MagpoLearner.loss_info(losses.cpu(), lrn.sys)
-    print(f"==== tc={tc} chunk={chunk}")
+    print(f"==== chunk={chunk}")
     k = 0
     for p in range(2):
         for m in range(2):
@@ -46,6 +44,5 @@ def run(tc: int, chunk: int):
 
 
 if __name__ == "__main__":
-    for tc in (0, 1):
-        for chunk in (0, 3):
-            run(tc, chunk)
+    for chunk in (0, 3):
+        run(chunk)

@@ -1,8 +1,6 @@
 #!/usr/bin/env python
-"""Bisect of the first-update deviation at a BASELINE config (tools/tolerance_control.py): gradients of the first minibatch of update 0
-of the CUDA path against the fp32 / fp64 oracle, per tensor, with the tensor-core GEMMs / persistent GRU scans / chunkwise retention
-switched off one at a time. Usage (GPU box): python tools/diag_update0.py [coordsum|lbf]"""
-import copy
+"""First-update deviation at a BASELINE config (tools/tolerance_control.py): per optimiser step of update 0, the learner's gradient
+against the fp32 oracle's and its parameters against the oracle's optimiser. Usage (GPU box): python tools/diag_update0.py [coordsum|lbf]"""
 import os
 import sys
 
@@ -13,46 +11,15 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 from gpu_util import baseline_case  # noqa: E402
-from magpo_b200 import _lib as L  # noqa: E402
 from magpo_b200.learner import param_views  # noqa: E402
 from oracle import learner as olr  # noqa: E402
 
 env = sys.argv[1] if len(sys.argv) > 1 else "coordsum"
 torch.set_num_threads(os.cpu_count() or 1)
 dev = torch.device("cuda:0")
-lib = L.lib()
-spec, ncfg, osys, state, lrn0 = baseline_case(env, dev)
-s64 = copy.deepcopy(state)
-rec32, rec64 = {}, {}
+spec, ncfg, osys, state, _ = baseline_case(env, dev)
+rec32 = {}
 olr.update_step(state, spec, ncfg, osys, record=rec32)
-olr.update_step(s64, spec, ncfg, osys, record=rec64, dtype=torch.float64)
-g32, a32 = rec32["grads"][0]
-g64, a64 = rec64["grads"][0]
-
-
-def report(tag, gp, ap):
-    rows = []
-    for pre, mine, r32, r64 in (("g/", gp, g32, g64), ("a/", ap, a32, a64)):
-        for k, r in r64.items():
-            sc = max(float(np.abs(r).max()), 1e-30)
-            rows.append((float(np.abs(mine[k].cpu().numpy() - r).max()) / sc, float(np.abs(r32[k] - r).max()) / sc, sc, pre + k))
-    rows.sort(reverse=True)
-    print(f"=== {tag}: worst gradient tensors of minibatch 0 (|cuda - o64| / max|g|, |o32 - o64| / max|g|, max|g|)")
-    for r in rows[:6]:
-        print("    %.2e  %.2e  %.2e  %s" % r)
-
-
-for tag, tc, gru, scan in (("default", 1, 0, 0), ("tensor cores off", 0, 0, 0), ("gru stepwise", 1, 1, 0), ("retention scan", 1, 0, 1),
-                           ("all off", 0, 1, 1)):
-    lib.magpo_set_tensor_cores(tc)
-    lib.magpo_debug_force_gru_stepwise(gru)
-    lib.magpo_debug_force_retention_scan(scan)
-    _, _, _, _, lrn = baseline_case(env, dev)
-    lrn.rollout(); lrn.gae(); lrn.epoch_indices(True); lrn.minibatch_grads(0)
-    torch.cuda.synchronize()
-    g = lrn.grads.clone()
-    report(tag, param_views(g[:lrn.n_g], lrn.g_table), param_views(g[lrn.n_g:lrn.n_g + lrn.n_a], lrn.a_table))
-lib.magpo_set_tensor_cores(1); lib.magpo_debug_force_gru_stepwise(0); lib.magpo_debug_force_retention_scan(0)
 
 # every optimiser step of update 0: gradient of step k (CUDA vs the fp32 oracle's), then the parameters after the step against the
 # oracle's optimiser replayed on the oracle's recorded gradients from the same initial parameters
