@@ -548,3 +548,6 @@ int retention_chunk_bwd(cudaStream_t s, int T, int N, int A, float kappa, bool c
 }
 
 }  // namespace magpo
+
+// Host-only: timesteps per chunk the chunkwise kernels launch with for A agents (tests assert which chunk geometry a case covers).
+extern "C" int magpo_debug_retention_chunk_len(int A) { return magpo::retention_chunk_len(A); }
