@@ -518,6 +518,107 @@ XLA_FFI_DEFINE_HANDLER_SYMBOL(magpo_ffi_clip_adam, ClipAdam,
                               ffi::Ffi::Bind() STREAM_ARGS_RETS.Attr<int64_t>("n").Attr<float>("grad_scale").Attr<float>("lr").Attr<int32_t>("decay_period")
                                   .Attr<int32_t>("num_updates").Attr<float>("max_norm"));
 
+// ------------------------------------------------------------------ rec_ippo (mava/systems/ppo/anakin/rec_ippo.py)
+// The workspaces are result buffers sized on the Python side by calling the entry point itself with workspace == NULL.
+// Rollout. operands: actor f32[n_a], critic f32[n_c], then in-out: key u32[2], the env state arrays, policy_h, critic_h f32[B,A,H], the 4
+// observation arrays of the trajectory; results: the aliased in-outs in the same order, the 11 timestep arrays, the remaining 12 trajectory
+// arrays (action ... last_value; sable_h0 x3 are 1-element placeholders), critic_h0 f32[B,A,H], workspace
+ffi::Error IppoRollout(cudaStream_t s, Args a, Rets r, NET_ATTR_PARAMS, SYS_ATTR_PARAMS, int32_t env_kind, int32_t e0, int32_t e1, int32_t e2,
+                       int32_t e3, int32_t e4, int32_t e5, int32_t e6, int32_t e7, int32_t carry_over) {
+  Unpack u(a, r, s);
+  const MagpoNetCfg net = net_cfg(NET_ATTR_ARGS);
+  const MagpoSysCfg sys = sys_cfg(SYS_ATTR_ARGS);
+  const int32_t env_attr[8] = {e0, e1, e2, e3, e4, e5, e6, e7};
+  const float* actor = u.in<float>();
+  const float* critic = u.in<float>();
+  uint32_t* key = u.inout<uint32_t>();
+  MagpoCoordSumState cs; MagpoLbfState lbf; MagpoRwareState rw;
+  void* env_state = nullptr;
+  if (env_kind == MAGPO_ENV_COORDSUM) { u.inout_struct(&cs); env_state = &cs; }
+  else if (env_kind == MAGPO_ENV_LBF) { u.inout_struct(&lbf); env_state = &lbf; }
+  else if (env_kind == MAGPO_ENV_RWARE) { u.inout_struct(&rw); env_state = &rw; }
+  else return ffi::Error::InvalidArgument("magpo_ffi_ippo_rollout: env_kind");
+  float* policy_h = u.inout<float>();
+  float* critic_h = u.inout<float>();
+  MagpoTrajectory traj;
+  u.inout_struct(&traj, 0, 4);
+  MagpoTimeStep ts;
+  u.out_struct(&ts);
+  u.out_struct(&traj, 4, 12);
+  float* critic_h0 = u.out<float>();
+  size_t ws_bytes = 0;
+  void* ws = u.out<char>(&ws_bytes);
+  if (!u.ok) return u.bad();
+  return status(magpo_ippo_rollout(context(), s, &net, &sys, env_kind, env_attr, env_state, ts, actor, critic, key, policy_h, critic_h, traj,
+                                   critic_h0, carry_over, ws, &ws_bytes), "magpo_ippo_rollout");
+}
+XLA_FFI_DEFINE_HANDLER_SYMBOL(magpo_ffi_ippo_rollout, IppoRollout,
+                              ffi::Ffi::Bind() STREAM_ARGS_RETS NET_ATTR_BIND SYS_ATTR_BIND.Attr<int32_t>("env_kind").Attr<int32_t>("env_cfg0")
+                                  .Attr<int32_t>("env_cfg1").Attr<int32_t>("env_cfg2").Attr<int32_t>("env_cfg3").Attr<int32_t>("env_cfg4")
+                                  .Attr<int32_t>("env_cfg5").Attr<int32_t>("env_cfg6").Attr<int32_t>("env_cfg7").Attr<int32_t>("carry_over"));
+
+// Epoch shuffle. operands: key u32[2] (in-out); results: key (aliased), perm i32[E], env_index, env_slot i32[M*U*N], workspace
+ffi::Error IppoEpochIndices(cudaStream_t s, Args a, Rets r, SYS_ATTR_PARAMS) {
+  Unpack u(a, r, s);
+  const MagpoSysCfg sys = sys_cfg(SYS_ATTR_ARGS);
+  uint32_t* key = u.inout<uint32_t>();
+  int32_t* perm = u.out<int32_t>();
+  int32_t* env_index = u.out<int32_t>();
+  int32_t* env_slot = u.out<int32_t>();
+  size_t ws_bytes = 0;
+  void* ws = u.out<char>(&ws_bytes);
+  if (!u.ok) return u.bad();
+  return status(magpo_ippo_epoch_indices(s, &sys, key, perm, env_index, env_slot, ws, &ws_bytes), "magpo_ippo_epoch_indices");
+}
+XLA_FFI_DEFINE_HANDLER_SYMBOL(magpo_ffi_ippo_epoch_indices, IppoEpochIndices, ffi::Ffi::Bind() STREAM_ARGS_RETS SYS_ATTR_BIND);
+
+// Gather. operands: the 16 trajectory arrays, critic_h0 f32[B,A,H], advantages, targets f32[T,B,A], env_index i32[n_env];
+// results: the 13 minibatch arrays (sable_h0 x3 are placeholders), critic_h0 f32[n_env,A,H]
+ffi::Error IppoPackMinibatch(cudaStream_t s, Args a, Rets r, NET_ATTR_PARAMS, SYS_ATTR_PARAMS, int32_t n_env) {
+  Unpack u(a, r, s);
+  const MagpoNetCfg net = net_cfg(NET_ATTR_ARGS);
+  const MagpoSysCfg sys = sys_cfg(SYS_ATTR_ARGS);
+  MagpoTrajectory traj;
+  u.in_struct(&traj);
+  const float* critic_h0 = u.in<float>();
+  const float* adv = u.in<float>();
+  const float* tgt = u.in<float>();
+  const int32_t* env_index = u.in<int32_t>();
+  MagpoMinibatch mb;
+  minibatch_from(u, &mb, rollout_length, n_env, true);
+  float* out_critic_h0 = u.out<float>();
+  if (!u.ok) return u.bad();
+  return status(magpo_ippo_pack_minibatch(s, &net, &sys, traj, critic_h0, adv, tgt, env_index, n_env, mb, out_critic_h0),
+                "magpo_ippo_pack_minibatch");
+}
+XLA_FFI_DEFINE_HANDLER_SYMBOL(magpo_ffi_ippo_pack_minibatch, IppoPackMinibatch,
+                              ffi::Ffi::Bind() STREAM_ARGS_RETS NET_ATTR_BIND SYS_ATTR_BIND.Attr<int32_t>("n_env"));
+
+// actor_grad_fn + critic_grad_fn. operands: actor, critic, the 13 minibatch arrays, critic_h0 f32[N,A,H], env_slot i32[N], adv_stats f32[U,2],
+// grads (in-out); results: grads f32[n_a+n_c+8] (aliased: accumulated into), workspace
+ffi::Error IppoMinibatchGrads(cudaStream_t s, Args a, Rets r, NET_ATTR_PARAMS, SYS_ATTR_PARAMS, int32_t T, int32_t N, float inv_tokens,
+                              int32_t reduce_grads) {
+  Unpack u(a, r, s);
+  const MagpoNetCfg net = net_cfg(NET_ATTR_ARGS);
+  const MagpoSysCfg sys = sys_cfg(SYS_ATTR_ARGS);
+  const float* actor = u.in<float>();
+  const float* critic = u.in<float>();
+  MagpoMinibatch mb;
+  minibatch_from(u, &mb, T, N, false);
+  const float* critic_h0 = u.in<float>();
+  const int32_t* env_slot = u.in<int32_t>();
+  const float* stats = u.in<float>();
+  float* grads = u.inout<float>();
+  size_t ws_bytes = 0;
+  void* ws = u.out<char>(&ws_bytes);
+  if (!u.ok) return u.bad();
+  return status(magpo_ippo_minibatch_grads(context(), s, &net, &sys, actor, critic, mb, critic_h0, env_slot, stats, inv_tokens, grads,
+                                           reduce_grads, ws, &ws_bytes), "magpo_ippo_minibatch_grads");
+}
+XLA_FFI_DEFINE_HANDLER_SYMBOL(magpo_ffi_ippo_minibatch_grads, IppoMinibatchGrads,
+                              ffi::Ffi::Bind() STREAM_ARGS_RETS NET_ATTR_BIND SYS_ATTR_BIND.Attr<int32_t>("T").Attr<int32_t>("N").Attr<float>("inv_tokens")
+                                  .Attr<int32_t>("reduce_grads"));
+
 // ------------------------------------------------------------------ data-parallel exchange (lax.pmean(..., "device"), :399-409)
 // The communicator is created on the host (magpo_ffi_comm_attach below) once per process; this handler sums a buffer over the ranks.
 // operands: buf f32[n] (in-out); results: buf (aliased)

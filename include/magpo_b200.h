@@ -88,7 +88,8 @@ typedef struct MagpoSysCfg {
  * Parameters of one network live in ONE flat float32 buffer; the tensors are laid out in the
  * canonical order reported here, named by their flax tree path (SURVEY.md Appendix A8/A9),
  * e.g. "encoder/encoder_block_0/retn/retention_heads_0/w_q".  which: 0 = guider (SableNetwork,
- * networks/sable_network.py:346), 1 = learner (RecurrentActor, networks/base.py:152). */
+ * networks/sable_network.py:346), 1 = learner (RecurrentActor, networks/base.py:152), 2 = rec_ippo's critic
+ * (RecurrentValueNet, networks/base.py:187-226: the learner's layout at action_dim 1, head "Dense_0"). */
 int64_t magpo_param_count(const MagpoNetCfg* cfg, int which);
 int32_t magpo_param_num_tensors(const MagpoNetCfg* cfg, int which);
 /* name -> static string; shape: up to 2 dims (dim1 == 0 for vectors); ld = row stride in floats: tensors that
@@ -381,6 +382,45 @@ int magpo_clip_adam(magpo_stream_t s, int64_t n, float* params, const float* gra
 int magpo_clip_adam_sched(magpo_stream_t s, int64_t n, float* params, const float* grads, float* mu,
                           float* nu, int32_t* count, float grad_scale, float lr, int32_t decay_period,
                           int32_t num_updates, float max_norm, float* scratch);
+
+/* ------------------------------------------------------------------ rec_ippo
+ * mava/systems/ppo/anakin/rec_ippo.py: recurrent IPPO, the learner's GRU actor (parameters `which` 1) beside a GRU critic (RecurrentValueNet,
+ * parameters `which` 2), trained with rec_sable's clipped PPO + clipped value loss. The same conventions as above; each entry point sizes its
+ * own workspace (CUB style): with workspace == NULL it writes the bytes it needs to *workspace_bytes and returns MAGPO_OK, otherwise
+ * *workspace_bytes is the capacity of `workspace`. The update between these calls is magpo_gae, magpo_adv_stats and magpo_clip_adam_sched. */
+
+/* lax.scan(_env_step, length=T) + the bootstrap value for B = U*E envs (slot-major, every slot on the same key), per step:
+ * key, policy_key = split(key); actor and critic each take (obs_t, last_done) and reset their own carry where last_done is set; the action
+ * is Categorical(masked logits).sample(seed=policy_key) with tfp's noise layout (element (e, agent, j) uses counter (e*A + agent)*a + j,
+ * e = b mod E); env.step. The bootstrap value is the critic on the final observation, final critic state and last done (its new state
+ * discarded, no key consumed): `key` advances by exactly T splits. traj.value gets the critic's values, traj.sable_h0 is not used;
+ * traj.policy_h0 / critic_h0 [B,A,H] receive the actor's / critic's state before the first step. policy_h / critic_h [B,A,H] in/out.
+ * Observation slots and carry_over as for magpo_rollout. */
+int magpo_ippo_rollout(MagpoContext* ctx, magpo_stream_t s, const MagpoNetCfg* net, const MagpoSysCfg* sys, int env_kind,
+                       const void* env_cfg, void* env_state, MagpoTimeStep ts, const float* actor, const float* critic, uint32_t* key,
+                       float* policy_h, float* critic_h, MagpoTrajectory traj, float* critic_h0, int32_t carry_over, void* workspace,
+                       size_t* workspace_bytes);
+
+/* Per-epoch shuffle: key, shuffle_key, _ = split(key, 3) (key advanced in place); perm = permutation(shuffle_key, E); for every minibatch
+ * m, slot u, position j (layout [M][U][N], N = E/M): env_index = u*E + perm[m*N + j], env_slot = u. No agent shuffle and no permutation
+ * carried across epochs. */
+int magpo_ippo_epoch_indices(magpo_stream_t s, const MagpoSysCfg* sys, uint32_t* key, int32_t* perm /*[E]*/, int32_t* env_index,
+                             int32_t* env_slot, void* workspace, size_t* workspace_bytes);
+
+/* Gathers n_env envs of the trajectory, agents in order, into `out` (out.sable_h0 unused) and both stored t = 0 hidden states by
+ * env_index: traj.policy_h0 -> out.policy_h0, critic_h0 [B,A,H] -> out_critic_h0 [n_env,A,H]. */
+int magpo_ippo_pack_minibatch(magpo_stream_t s, const MagpoNetCfg* net, const MagpoSysCfg* sys, MagpoTrajectory traj,
+                              const float* critic_h0, const float* advantages, const float* targets, const int32_t* env_index, int32_t n_env,
+                              MagpoMinibatch out, float* out_critic_h0);
+
+/* actor_grad_fn + critic_grad_fn for the envs held in `mb` (critic_h0 [mb.N,A,H]); env_slot / adv_stats / inv_tokens as for
+ * magpo_minibatch_grads. grads [n_actor + n_critic + 8], ACCUMULATED into: actor grads | critic grads | {-, actor_loss, entropy,
+ * value_loss, 0, -, actor_loss, 0} (the slots of magpo_minibatch_grads with rec_sable's values). With reduce_grads != 0 and a communicator
+ * attached to the context, the whole buffer is sum-all-reduced over the ranks at the end. */
+int magpo_ippo_minibatch_grads(MagpoContext* ctx, magpo_stream_t s, const MagpoNetCfg* net, const MagpoSysCfg* sys, const float* actor,
+                               const float* critic, MagpoMinibatch mb, const float* critic_h0, const int32_t* env_slot,
+                               const float* adv_stats, float inv_tokens, float* grads, int32_t reduce_grads, void* workspace,
+                               size_t* workspace_bytes);
 
 /* ------------------------------------------------------------------ data-parallel exchange
  * `jax.lax.pmean(..., "device")` (rec_magpo.py:399-409) as NCCL all-reduces over NVLink / NVSwitch, one process per GPU. libnccl.so.2

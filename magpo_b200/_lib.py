@@ -174,6 +174,14 @@ def call(name: str, *args) -> None:
     check(getattr(lib(), name)(*args), name)
 
 
+def workspace_bytes(name: str, *args) -> int:
+    """The workspace size of an entry point that answers the CUB-style query (the rec_ippo ones): `args` are every argument before
+    `workspace`; called with workspace NULL it writes the size to its `size_t* workspace_bytes`."""
+    n = C.c_size_t(0)
+    check(getattr(lib(), name)(*args, None, C.byref(n)), name)
+    return int(n.value)
+
+
 def stream_ptr(stream=None) -> vp:
     import torch
 

@@ -64,7 +64,7 @@ pack_rows_kernel(int T, int B, int A, int d, int a, int n_env, MagpoTrajectory t
     const int i = (int)(row % A);
     const int n = (int)((row / A) % n_env);
     const int t = (int)(row / ((int64_t)A * n_env));
-    const int b = env_index[n], ai = agent_perm[i];
+    const int b = env_index[n], ai = agent_perm ? agent_perm[i] : i;
     const int64_t src = ((int64_t)t * B + b) * A + ai;
     for (int c = lane; c < d; c += 32) o_view[row * d + c] = tr.agents_view[src * d + c];
     for (int c = lane; c < a; c += 32) o_mask[row * a + c] = tr.action_mask[src * a + c];
@@ -94,7 +94,7 @@ pack_rows_narrow_kernel(int T, int B, int A, int d, int a, int n_env, MagpoTraje
     const int i = (int)(row % A);
     const int n = (int)((row / A) % n_env);
     const int t = (int)(row / ((int64_t)A * n_env));
-    const int b = __ldg(env_index + n), ai = __ldg(agent_perm + i);
+    const int b = __ldg(env_index + n), ai = agent_perm ? __ldg(agent_perm + i) : i;
     const int64_t src = ((int64_t)t * B + b) * A + ai;
     const int32_t st = tr.step_count[src], ac = tr.action[src];
     const float va = tr.value[src], lp = tr.log_prob[src], ad = adv[src], tg = tgt[src];
@@ -204,6 +204,30 @@ __global__ void mask_logits_kernel(int64_t n, const uint8_t* __restrict__ mask, 
 }
 
 }  // namespace
+
+int epoch_index(cudaStream_t s, int E, int U, int M, const int32_t* batch_perm, int32_t* hs_perm, int first_epoch, int32_t* hs_perm_new,
+                int32_t* env_index, int32_t* hs_index, int32_t* env_slot) {
+  const int total = M * U * (E / M);
+  epoch_index_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, s>>>(E, U, M, batch_perm, hs_perm, first_epoch, hs_perm_new, env_index,
+                                                                   hs_index, env_slot);
+  MAGPO_LAUNCH_OK();
+  return MAGPO_OK;
+}
+
+int pack_rows(cudaStream_t s, const MagpoNetCfg* net, const MagpoSysCfg* sys, const MagpoTrajectory& traj, const float* advantages,
+              const float* targets, const int32_t* env_index, const int32_t* agent_perm, int n_env, const MagpoMinibatch& out) {
+  const int A = net->n_agents, T = sys->rollout_length, B = sys->update_batch_size * sys->num_envs;
+  const int64_t R = (int64_t)T * n_env * A;
+  const bool narrow = net->obs_dim <= 16;
+  (narrow ? pack_rows_narrow_kernel : pack_rows_kernel)<<<(unsigned)std::min<int64_t>(ceil_div(R, narrow ? 256 : 8), (int64_t)kNumSMs * 16), 256, 0, s>>>(
+      T, B, A, net->obs_dim, net->action_dim, n_env, traj, advantages, targets, env_index, agent_perm,
+      const_cast<float*>(out.agents_view), const_cast<uint8_t*>(out.action_mask), const_cast<int32_t*>(out.step_count),
+      const_cast<uint8_t*>(out.done), const_cast<int32_t*>(out.action), const_cast<float*>(out.value),
+      const_cast<float*>(out.log_prob), const_cast<float*>(out.advantages), const_cast<float*>(out.targets));
+  MAGPO_LAUNCH_OK();
+  return MAGPO_OK;
+}
+
 }  // namespace magpo
 
 using namespace magpo;
@@ -225,10 +249,7 @@ int magpo_epoch_indices(magpo_stream_t s_, const MagpoSysCfg* sys, int32_t A, ui
   MAGPO_LAUNCH_OK();
   MAGPO_TRY(magpo_prng_permutation(s_, sub, E, batch_perm, pscr));
   MAGPO_TRY(magpo_prng_permutation(s_, sub + 2, A, agent_perm, pscr));
-  const int total = M * U * (E / M);
-  epoch_index_kernel<<<(unsigned)ceil_div(total, 256), 256, 0, s>>>(E, U, M, batch_perm, hs_perm, first_epoch, hs_new,
-                                                                   env_index, hs_index, env_slot);
-  MAGPO_LAUNCH_OK();
+  MAGPO_TRY(epoch_index(s, E, U, M, batch_perm, hs_perm, first_epoch, hs_new, env_index, hs_index, env_slot));
   MAGPO_CUDA_OK(cudaMemcpyAsync(hs_perm, hs_new, sizeof(int32_t) * E, cudaMemcpyDeviceToDevice, s));
   return MAGPO_OK;
 }
@@ -246,16 +267,10 @@ int magpo_pack_minibatch(magpo_stream_t s_, const MagpoNetCfg* net, const MagpoS
   if (!sys || !advantages || !targets || !env_index || !hs_index || !agent_perm || n_env < 1) return MAGPO_ERR_ARG;
   if (out.T != sys->rollout_length || out.N != n_env) return MAGPO_ERR_ARG;
   cudaStream_t s = as_stream(s_);
-  const int A = net->n_agents, T = sys->rollout_length, B = sys->update_batch_size * sys->num_envs;
+  const int A = net->n_agents, T = sys->rollout_length;
   const int64_t R = (int64_t)T * n_env * A;
   ProfScope ps(PROF_PACK, s, 2.0 * (double)R * (4.0 * net->obs_dim + net->action_dim + 24.0) + 2.0 * n_env * (3 * 16384.0 + 512.0 * A));
-  const bool narrow = net->obs_dim <= 16;
-  (narrow ? pack_rows_narrow_kernel : pack_rows_kernel)<<<(unsigned)std::min<int64_t>(ceil_div(R, narrow ? 256 : 8), (int64_t)kNumSMs * 16), 256, 0, s>>>(
-      T, B, A, net->obs_dim, net->action_dim, n_env, traj, advantages, targets, env_index, agent_perm,
-      const_cast<float*>(out.agents_view), const_cast<uint8_t*>(out.action_mask), const_cast<int32_t*>(out.step_count),
-      const_cast<uint8_t*>(out.done), const_cast<int32_t*>(out.action), const_cast<float*>(out.value),
-      const_cast<float*>(out.log_prob), const_cast<float*>(out.advantages), const_cast<float*>(out.targets));
-  MAGPO_LAUNCH_OK();
+  MAGPO_TRY(pack_rows(s, net, sys, traj, advantages, targets, env_index, agent_perm, n_env, out));
   pack_hidden_kernel<<<n_env, 256, 0, s>>>(A, n_env, (int)(NetShape::of(net).state_elems() / 4), traj.policy_h0, traj.sable_h0.encoder, traj.sable_h0.decoder_self,
                                            traj.sable_h0.decoder_cross, env_index, hs_index, agent_perm,
                                            const_cast<float*>(out.policy_h0), out.sable_h0.encoder,
@@ -504,8 +519,10 @@ static int guider_table(const MagpoNetCfg* net, ParamEntry* out) {
   return n;
 }
 
-static int actor_table(const MagpoNetCfg* net, ParamEntry* out) {
-  const int d = net->obs_dim, a = net->action_dim;
+// which 1: the learner's RecurrentActor; which 2: rec_ippo's critic, RecurrentValueNet (networks/base.py:187-226): the same torsos and
+// GRU with a Dense(1) head and no action mask (the actor's layout at a = 1)
+static int actor_table(const MagpoNetCfg* net, ParamEntry* out, int which) {
+  const int d = net->obs_dim, a = which == 2 ? 1 : net->action_dim;
   ActorP p = ActorP::bind(reinterpret_cast<float*>(sizeof(float)), d, a);
   auto off = [](const float* q) { return (int64_t)(reinterpret_cast<uintptr_t>(q) / sizeof(float)) - 1; };
   int n = 0;
@@ -527,8 +544,10 @@ static int actor_table(const MagpoNetCfg* net, ParamEntry* out) {
   add("ScannedRNN_0/GRUCell_0/hn/bias", p.bhn, 0, kH, 0, 1);
   add("post_torso/Dense_0/kernel", p.post_w, 0, kH, kH, kH);
   add("post_torso/Dense_0/bias", p.post_b, 0, kH, 0, 1);
-  add("action_head/Dense_0/kernel", p.head_w, 0, kH, a, a);
-  add("action_head/Dense_0/bias", p.head_b, 0, a, 0, 1);
+  // the critic's head is created directly in RecurrentValueNet's compact body, so its flax path is the bare auto-name (from memory)
+  const bool critic = which == 2;
+  add(critic ? "Dense_0/kernel" : "action_head/Dense_0/kernel", p.head_w, 0, kH, a, a);
+  add(critic ? "Dense_0/bias" : "action_head/Dense_0/bias", p.head_b, 0, a, 0, 1);
   return n;
 }
 
@@ -544,13 +563,13 @@ int64_t magpo_param_count(const MagpoNetCfg* net, int which) {
   if (check_net(net) != MAGPO_OK) return -1;
   if (which == 0 && !NetShape::of(net).is_default()) return GuiderG::bind(nullptr, NetShape::of(net)).total;
   return which == 0 ? GuiderP::bind(nullptr, net->obs_dim, net->action_dim).total
-                    : ActorP::bind(nullptr, net->obs_dim, net->action_dim).total;
+                    : ActorP::bind(nullptr, net->obs_dim, which == 2 ? 1 : net->action_dim).total;
 }
 
 int32_t magpo_param_num_tensors(const MagpoNetCfg* net, int which) {
   if (check_net(net) != MAGPO_OK) return -1;
   if (which == 0 && !NetShape::of(net).is_default()) return (int32_t)general_table(net).size();
-  return which == 0 ? guider_table(net, nullptr) : actor_table(net, nullptr);
+  return which == 0 ? guider_table(net, nullptr) : actor_table(net, nullptr, which);
 }
 
 int magpo_param_tensor(const MagpoNetCfg* net, int which, int32_t index, const char** name, int64_t* offset,
@@ -564,7 +583,7 @@ int magpo_param_tensor(const MagpoNetCfg* net, int which, int32_t index, const c
     return MAGPO_OK;
   }
   ParamEntry tab[64];
-  const int n = which == 0 ? guider_table(net, tab) : actor_table(net, tab);
+  const int n = which == 0 ? guider_table(net, tab) : actor_table(net, tab, which);
   if (index < 0 || index >= n || !name || !offset || !dim0 || !dim1 || !ld) return MAGPO_ERR_ARG;
   *name = tab[index].name;
   *offset = tab[index].offset;

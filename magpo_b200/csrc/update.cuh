@@ -13,6 +13,13 @@ int magpo_losses(cudaStream_t s, int64_t R, int N, int A, int a, const MagpoSysC
                  const float* adv, const float* value, const float* value_old, const float* targets,
                  const int32_t* env_slot, const float* stats, float* dlg, float* dll, float* dvalue, float* loss_sums);
 
+// env_index / hs_index / env_slot of every minibatch of an epoch, laid out [M][U][E/M] (rec_magpo.py:439-451)
+int epoch_index(cudaStream_t s, int E, int U, int M, const int32_t* batch_perm, int32_t* hs_perm, int first_epoch, int32_t* hs_perm_new,
+                int32_t* env_index, int32_t* hs_index, int32_t* env_slot);
+// The per-token rows of n_env envs of the trajectory, time-major [T, n_env, A, ...]; agent_perm NULL: agents in order.
+int pack_rows(cudaStream_t s, const MagpoNetCfg* net, const MagpoSysCfg* sys, const MagpoTrajectory& traj, const float* advantages,
+              const float* targets, const int32_t* env_index, const int32_t* agent_perm, int n_env, const MagpoMinibatch& out);
+
 // guider / learner work may run on forked streams (magpo_debug_set_overlap)
 bool nets_overlap_enabled();
 

@@ -212,3 +212,13 @@ def flax_init_actor(actor_net_key, obs_dim: int, action_dim: int, device="cuda:0
     p["post_torso/Dense_0/kernel"] = _flax_orthogonal(_flax_param_key(actor_net_key, ("post_torso", "Dense_0"), 0), (H, H), sq2, device)
     p["action_head/Dense_0/kernel"] = _flax_orthogonal(_flax_param_key(actor_net_key, ("action_head", "Dense_0"), 0), (H, action_dim), 0.01, device)
     return p
+
+
+def flax_init_critic(critic_net_key, obs_dim: int, device="cuda:0", H: int = 128) -> dict:
+    """RecurrentValueNet.init(critic_net_key, ...) (rec_ippo.py learner_setup; networks/base.py:187-226): the actor's torsos and GRU
+    with flax_init_actor's initialisers, and a Dense(1) head with orthogonal(1.0) under the path the parameter table names."""
+    p = flax_init_actor(critic_net_key, obs_dim, 1, device, H)
+    del p["action_head/Dense_0/kernel"], p["action_head/Dense_0/bias"]
+    p["Dense_0/kernel"] = _flax_orthogonal(_flax_param_key(critic_net_key, ("Dense_0",), 0), (H, 1), 1.0, device)
+    p["Dense_0/bias"] = np.zeros(1, np.float32)
+    return p

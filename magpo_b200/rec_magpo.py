@@ -150,6 +150,20 @@ def make_env(config: Config):
     raise NotImplementedError(f"{name}: only CoordSum, LevelBasedForaging and RobotWarehouse dynamics are built")
 
 
+def check_torsos(network, which: str, hidden: int) -> None:
+    """`network.<which>.{pre,post}_torso` must be the default MLPTorso the GRU kernels are built for; anything else raises."""
+    an = network.get(which)
+    if an is None:
+        return
+    for name in ("pre_torso", "post_torso"):
+        t = an.get(name)
+        if t is None:
+            continue
+        if [int(x) for x in t.layer_sizes] != [hidden] or bool(t.get("use_layer_norm", False)) or t.get("activation", "relu") != "relu":
+            raise NotImplementedError(f"network.{which}.{name}: only one Dense({hidden}) + relu layer without layer norm is built "
+                                      "(RecurrentActor of configs/network/magpo.yaml:19-31)")
+
+
 def _network_config(config: Config, env) -> NetworkConfig:
     """`config.network` (configs/network/magpo.yaml) + env dims -> the shapes the kernels are built for. Everything the reference
     reads is read here; a value the kernels do not cover raises instead of being silently ignored (the library's own
@@ -159,15 +173,7 @@ def _network_config(config: Config, env) -> NetworkConfig:
     if not bool(config.system.get("add_agent_id", True)):
         raise NotImplementedError("system.add_agent_id=False: the env kernels emit the AgentIDWrapper observation only")
     hidden = int(n.get("hidden_state_dim", 128))
-    an = n.get("actor_network")
-    if an is not None:
-        for name in ("pre_torso", "post_torso"):
-            t = an.get(name)
-            if t is None:
-                continue
-            if [int(x) for x in t.layer_sizes] != [hidden] or bool(t.get("use_layer_norm", False)) or t.get("activation", "relu") != "relu":
-                raise NotImplementedError(f"network.actor_network.{name}: only one Dense({hidden}) + relu layer without layer norm is built "
-                                          "(RecurrentActor of configs/network/magpo.yaml:19-31)")
+    check_torsos(n, "actor_network", hidden)
     # memory_config.timestep_chunk_size: chunking the sequence is mathematically exact (tests/test_oracle.py
     # ::test_timestep_chunking_is_exact), the kernels always run their own chunked scan, so any value is accepted.
     net = NetworkConfig(env.num_agents, env.obs_dim, env.action_dim, env.time_limit, embed_dim=int(nc.embed_dim), n_head=int(nc.n_head),
