@@ -36,6 +36,7 @@ constexpr int TC_CHUNK_BYTES = TC_BM * TC_KC * 4;  // 16 KiB
 constexpr int TC_CONV_THREADS = 256;               // warps 8..15
 constexpr int TC_THREADS = 256 + TC_CONV_THREADS;
 constexpr int TC_MAX_STAGES = 6;
+constexpr int kTnMaxRows = 8192;  // rows one gemm_tc_tn accumulator reduces (see gemm_tc_tn)
 constexpr uint32_t TC_SMEM_LIMIT = 227 * 1024;
 
 struct TcParams {
@@ -236,8 +237,8 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ 
 // Weight-gradient GEMM on the tensor cores:  dW[K,N] += X[M,K]^T @ dY[M,N]   (K in {64,128}; reduction over the rows).
 // Both operands are activations and are consumed exactly as they lie in memory: a [32 rows x 32 floats] TMA box is an
 // MN-major (M/N contiguous) 128B-swizzled UMMA operand whose 8-row groups are the K=8 steps of kind::tf32. Both operands are
-// split into TF32 hi/lo by the converter warps. Each CTA reduces a contiguous slab of rows into one TMEM accumulator and
-// adds it to dW with a TMA reduce-add, so the cross-CTA reduction needs no extra pass.
+// split into TF32 hi/lo by the converter warps. Each CTA reduces a contiguous slab of at most kTnMaxRows rows into one TMEM
+// accumulator and adds it to dW with a TMA reduce-add, so the cross-CTA reduction needs no extra pass.
 // rows per pipeline stage: 32, or 64 where the stage stays small (narrow K and N): the per-stage hand-overs (barrier round trips of the
 // producer / converter / MMA roles) cost the same for 16 KiB as for 48 KiB, and the narrow GEMMs were bound by them
 
@@ -574,7 +575,11 @@ int gemm_tc_tn(cudaStream_t s, int64_t M, int N, int K, const float* X, int ldx,
   const int n_tiles = N / p.BN;
   const int TN_RC = p.rc;
   const int64_t chunks = ceil_div(M, TN_RC);
-  const int gx = (int)std::max<int64_t>(1, std::min<int64_t>(chunks, kNumSMs / n_tiles));
+  // A TMEM accumulator takes at most kTnMaxRows rows: the tensor core's fp32 accumulation error grows with the length of the chain (one
+  // slab of 65 k rows put CoordSum's GRU weight gradients 2.7e-4 from float64), so long reductions run as several full waves of slabs.
+  const int64_t per_wave = std::max(1, kNumSMs / n_tiles);
+  const int64_t waves = ceil_div(chunks, per_wave * (kTnMaxRows / TN_RC));
+  const int gx = (int)std::max<int64_t>(1, std::min<int64_t>(chunks, per_wave * waves));
   p.rows_per_cta = ceil_div(chunks, gx) * TN_RC;
   CUtensorMap tmX, tmDY, tmDW;
   // boxes of [32 rows x 32 floats] for the operands; the accumulator slab is [K rows x 32 floats]

@@ -177,7 +177,8 @@ def pos_encoding(step_count, D, dtype):
 
 
 def swiglu(p, pre, x):  # torsos.py:79-99
-    return (swish(x @ p[f"{pre}/W_gate"]) * (x @ p[f"{pre}/W_linear"])) @ p[f"{pre}/W_output"]
+    gate, linear = _rec(f"{pre}/gate", x @ p[f"{pre}/W_gate"]), _rec(f"{pre}/linear", x @ p[f"{pre}/W_linear"])
+    return _rec(f"{pre}/out", _rec(f"{pre}/hmid", swish(gate) * linear) @ p[f"{pre}/W_output"])
 
 
 # ----------------------------------------------------------------------------- retention
@@ -211,9 +212,9 @@ def _xi(ts_dones, kappa, n_agents, dtype):
 def simple_retention_chunk(p, pre, key, query, value, hstate, dones, kappa, n_agents, masked):
     """SimpleRetention.__call__ (retention.py:66-100), rec_sable branch."""
     B, C, _ = value.shape
-    q = query @ p[f"{pre}/w_q"]
-    k = key @ p[f"{pre}/w_k"]
-    v = value @ p[f"{pre}/w_v"]
+    q = _rec(f"{pre}/q", query @ p[f"{pre}/w_q"])
+    k = _rec(f"{pre}/k", key @ p[f"{pre}/w_k"])
+    v = _rec(f"{pre}/v", value @ p[f"{pre}/w_v"])
     kT = k.transpose(1, 2)
     ts_dones = dones[:, ::n_agents]
     D = _decay_matrix(ts_dones, kappa, n_agents, masked, value.dtype)
@@ -242,6 +243,8 @@ def msr(p, pre, cfg: NetCfg, key, query, value, hstate, step_count, masked, done
     if cfg.timestep_pe:
         pe = pos_encoding(step_count, D, value.dtype)
         key, query, value = key + pe, query + pe, value + pe
+    _rec(f"{pre}/key", key)
+    _rec(f"{pre}/query", query)
     outs, new_hs = [], []
     kap = cfg.kappas()
     for h in range(cfg.n_head):
@@ -255,21 +258,22 @@ def msr(p, pre, cfg: NetCfg, key, query, value, hstate, step_count, masked, done
     ret = torch.cat(outs, dim=-1)
     _rec(f"{pre}/ret", ret)
     ret = groupnorm_rows(ret.reshape(-1, cfg.head_size), p[f"{pre}/group_norm/scale"], p[f"{pre}/group_norm/bias"], cfg.n_head).reshape(ret.shape)
-    gated = _rec(f"{pre}/gated", swish(key @ p[f"{pre}/w_g"]) * ret)
+    gated = _rec(f"{pre}/gated", swish(_rec(f"{pre}/g", key @ p[f"{pre}/w_g"])) * ret)
     out = _rec(f"{pre}/out", gated @ p[f"{pre}/w_o"])
     return out, torch.stack(new_hs, dim=1)
 
 
 # ----------------------------------------------------------------------------- encoder / decoder
 def _head(p, pre, x):
-    h = gelu(x @ p[f"{pre}/layers_0/kernel"] + p[f"{pre}/layers_0/bias"])
+    h = gelu(_rec(f"{pre}/zh", x @ p[f"{pre}/layers_0/kernel"] + p[f"{pre}/layers_0/bias"]))
     h = rmsnorm(h, p[f"{pre}/layers_2/scale"])
     return h @ p[f"{pre}/layers_3/kernel"] + p[f"{pre}/layers_3/bias"]
 
 
 def encoder_apply(p, cfg: NetCfg, obs, hstate, step_count, dones=None):
     """Encoder.__call__ / Encoder.recurrent (sable_network.py:121-156). hstate [B,nh,nb,hs,hs]."""
-    x = gelu(rmsnorm(obs, p["encoder/obs_encoder/layers_0/scale"]) @ p["encoder/obs_encoder/layers_1/kernel"])
+    on = _rec("enc/on", rmsnorm(obs, p["encoder/obs_encoder/layers_0/scale"]))
+    x = gelu(_rec("enc/z0", on @ p["encoder/obs_encoder/layers_1/kernel"]))
     new_h = []
     for b in range(cfg.n_block):
         pre = f"encoder/encoder_block_{b}"
